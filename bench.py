@@ -15,8 +15,13 @@ rebuild of the derived parameter tables in the next step -- is inside the
 timed region, whatever --steps is.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 Prints one JSON line (see DESIGN.md section "Measurement" for every field).
+--dump-outputs DIR also writes what the timed headline run left its caller
+after the last timed step as DIR/<name>.npy (see dump_outputs); the inputs are
+seeded, so two builds run with the same arguments can be compared array by
+array.
 """
 import argparse
 import json
@@ -37,6 +42,7 @@ SWEEP_STEPS = N_SITES            # num_monte_carlo_sweeps (1) * num_sites
 SEED = 0xC65
 EPOCH_BATCHES = 50               # num_batches_per_epoch default (utils.py:132-138)
 L2_FLUSH_BYTES = 256 << 20
+DUMP_CONFIG_BYTES = 32 << 20     # --dump-outputs: larger walker sets are written as a seeded row sample
 
 # The BASELINE.json configurations (SURVEY.md 8(a) sizes, 8(d) synthetic inputs).
 # walkers = per GPU; max_steps bounds the timed steps of the slow configurations
@@ -76,7 +82,14 @@ def parse_args():
   ap.add_argument('--configs', default='C1,C3,C4,C5',
                   help='other BASELINE configurations to report as sub-results ("" = none)')
   ap.add_argument('--no-cpu-baseline', action='store_true')
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write the outputs of the last timed C2 step as DIR/<name>.npy (rank 0; --impl ours)')
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs applies to --impl ours')
+  return args
 
 
 def peaks():
@@ -571,6 +584,35 @@ def result_for(w, timing, steps, world, pk):
   return res
 
 
+def dump_outputs(w, timing, out_dir):
+  """Writes what an EnergyGradient run of workload `w` leaves its caller after
+  the last timed step (an epoch end) to out_dir/<name>.npy:
+    params          float32 [P]     parameters after the last Adam update
+    energy_stats    float64 [4]     sum E, sum E^2, walkers of the last epoch, 0
+    epoch_energies  float64 [E]     mean energy of every timed epoch
+    accepted_moves  float64 [1]     accepted Metropolis moves of this shard so far
+    configs         float32 [B, N]  walker configurations (+-1) of this shard
+  Walker sets above DUMP_CONFIG_BYTES are written as a fixed, seeded sample of
+  rows, and config_rows (float64) holds their indices."""
+  torch.cuda.synchronize()
+  configs = w.state.configs().cpu().numpy()
+  arrays = {
+      'params': w.ansatz.params.detach().cpu().numpy().astype(np.float32),
+      'energy_stats': w.host_stats.numpy().astype(np.float64),
+      'epoch_energies': np.asarray(timing['energies'], dtype=np.float64),
+      'accepted_moves': w.state.accept_count.cpu().numpy().astype(np.float64),
+  }
+  if configs.nbytes > DUMP_CONFIG_BYTES:
+    rows = np.sort(np.random.default_rng(SEED).choice(
+        configs.shape[0], DUMP_CONFIG_BYTES // configs[0].nbytes, replace=False))
+    configs = configs[rows]
+    arrays['config_rows'] = rows.astype(np.float64)
+  arrays['configs'] = configs.astype(np.float32)
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), np.ascontiguousarray(a))
+
+
 def parity_selfcheck(rank, world, dev):
   """N > 1: the all-reduced [sum O | sum E O | sum E, sum E^2, n | accepted
   moves] of `world` real shards equals the same quantities of `world` virtual
@@ -632,6 +674,8 @@ def run_ours(args, rank, world, local_rank):
   w = EnergyGradientWorkload('C2', B, rank, world, dev)
   timing = time_workload(w, args.steps, args.warmup, flush, world, dev,
                          clock_index=local_rank if rank == 0 else None)
+  if args.dump_outputs and rank == 0:     # before anything below steps the walkers again
+    dump_outputs(w, timing, args.dump_outputs)
   main = result_for(w, timing, args.steps, world, pk)
   P = w.ansatz.num_params
   # the same epochs with one launch per batch iteration (cgsvmc_batch_step), for comparison

@@ -36,3 +36,11 @@ def test_reference_arm_prints_one_json_line():
 def test_reference_arm_other_ranks_do_nothing():
   out = _run({'RANK': '1', 'WORLD_SIZE': '2', 'LOCAL_RANK': '1'})
   assert out.returncode == 0 and out.stdout.strip() == ''
+
+
+def test_bad_arguments_are_refused():
+  env = dict(os.environ, PYTHONPATH=REPO)
+  for extra in (['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'out']):
+    out = subprocess.run([sys.executable, os.path.join(REPO, 'bench.py')] + extra,
+                         capture_output=True, text=True, timeout=120, env=env)
+    assert out.returncode == 2 and out.stdout.strip() == '', extra
