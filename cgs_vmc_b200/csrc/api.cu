@@ -320,9 +320,6 @@ int cgsvmc_mc_steps(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, int32_t
   if (rbm2_supported(a, nullptr))
     return rbm2_mc_steps(const_cast<cgsvmc_ansatz*>(a), packed, B, n_steps, seed, walker_id0, step0,
                          accept_count, log_amp_out, (cudaStream_t)stream);
-  if (rbm_fast_supported(a))
-    return rbm_mc_steps(a, packed, B, n_steps, seed, walker_id0, step0, accept_count, log_amp_out,
-                        (cudaStream_t)stream);
   if (conv_tc_supported(a, nullptr))
     return conv_tc_mc_steps(const_cast<cgsvmc_ansatz*>(a), packed, B, n_steps, seed, walker_id0, step0,
                             accept_count, log_amp_out, (cudaStream_t)stream);
@@ -342,10 +339,6 @@ int cgsvmc_mc_steps_graph(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, i
   NvtxRange range("cgsvmc:K2 mc_steps_graph");
   if (a == nullptr) return invalid("ansatz handle is NULL");
   if (step_counter == nullptr) return invalid("mc_steps_graph: NULL step counter");
-  if (rbm_fast_supported(a) && !rbm2_supported(a, nullptr)) {
-    set_error("mc_steps_graph: not available on the first-generation RBM kernels");
-    return CGSVMC_ERR_UNSUPPORTED;
-  }
   cgsvmc_ansatz* am = const_cast<cgsvmc_ansatz*>(a);
   am->step_counter_dev = step_counter;
   const int rc = cgsvmc_mc_steps(a, packed, B, n_steps, seed, walker_id0, 0, accept_count, log_amp_out, stream);
@@ -425,7 +418,6 @@ int cgsvmc_weighted_grad_sum(const cgsvmc_ansatz* a, const uint64_t* packed, con
     }
     return CGSVMC_OK;
   }
-  if (rbm_fast_supported(a)) return rbm_grad(am, packed, weights, B, K, out, (cudaStream_t)stream);
   if (fc_tc_grad_supported(a)) return fc_tc_grad(am, packed, weights, B, K, out, (cudaStream_t)stream);
   if (conv_tc_grad_supported(a)) return conv_tc_grad(am, packed, weights, B, K, out, (cudaStream_t)stream);
   return net_grad(am, packed, weights, B, K, out, (cudaStream_t)stream);

@@ -739,23 +739,6 @@ bool tc_enabled() {
   return e == nullptr || atoi(e) != 0;
 }
 
-// Geometry and shared-memory plan; false when the network is outside the
-// tensor-core path (the SIMT tile kernels of net.cu take over).
-// CTAs per SM the kernels are planned for.  Two (default): each CTA runs its
-// layers as [MMAs of all tiles] -> [epilogue of all tiles]; with two resident
-// CTAs the tensor pipe works for one while the other runs its epilogue, and the
-// single weight buffer is refilled under the epilogue.  CGSVMC_CONV_TC_CTAS=1
-// selects the one-CTA plan (larger batches, double-buffered weights).
-int tc_ctas_wanted() {
-  const char* e = getenv("CGSVMC_CONV_TC_CTAS");
-  return e != nullptr && atoi(e) == 1 ? 1 : 2;
-}
-// CGSVMC_CONV_TC_IL=0 keeps the side-by-side layout (development comparison).
-bool tc_interleave_wanted() {
-  const char* e = getenv("CGSVMC_CONV_TC_IL");
-  return e == nullptr || atoi(e) != 0;
-}
-
 // rows / tiles / TMEM columns of a plan with G configurations
 void size_plan(TcDesc* t, int G) {
   t->G = G; t->GW = G * t->PW;
@@ -773,13 +756,17 @@ void size_plan(TcDesc* t, int G) {
 bool make_desc_plan(const cgsvmc_ansatz* a, size_t extra_bytes_per_cfg, size_t extra_fixed, int ctas, int il,
                     TcDesc* out);
 
-// Plans in order of measured throughput (C3 / C4 / 16x16, profiles/r02g_*): two
-// CTAs per SM before one (the tensor pipe of one works under the epilogue of the
-// other), and within that the interleaved layout before the side-by-side one.
+// Geometry and shared-memory plan; false when the network is outside the
+// tensor-core path (the SIMT tile kernels of net.cu take over).  Plans in order
+// of measured throughput (C3 / C4 / 16x16, profiles/r02g_*): two CTAs per SM
+// before one, and within that the interleaved layout before the side-by-side
+// one.  With two CTAs each runs its layers as [MMAs of all tiles] -> [epilogue
+// of all tiles]: the tensor pipe works for one while the other runs its
+// epilogue, and the single weight buffer is refilled under the epilogue.  The
+// one-CTA plan (larger batches, double-buffered weights) takes what two do not fit.
 bool make_desc_host(const cgsvmc_ansatz* a, size_t extra_bytes_per_cfg, size_t extra_fixed, TcDesc* out) {
-  const int max_ctas = tc_ctas_wanted();
-  for (int ctas = max_ctas; ctas >= 1; --ctas)
-    for (int il = tc_interleave_wanted() ? 1 : 0; il >= 0; --il)
+  for (int ctas = 2; ctas >= 1; --ctas)
+    for (int il = 1; il >= 0; --il)
       if (make_desc_plan(a, extra_bytes_per_cfg, extra_fixed, ctas, il, out)) return true;
   return false;
 }

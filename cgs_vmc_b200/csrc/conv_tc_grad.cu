@@ -60,7 +60,6 @@ struct GDesc {
   int PH, PW, G, GW;
   int rows_out, n_tiles, rows_total, kblocks;
   int n_tensor, wbuf_bytes, n_pairs;
-  int wg_m64;               // weight-gradient MMAs with M = 64 (accumulator rows 16 i + r in lanes 32 i + r)
   const __half *w1img, *wimg, *wimg_b;
   const float *bias, *wsum;
   int64_t w_off[kMaxL], b_off[kMaxL];
@@ -89,11 +88,11 @@ __host__ __device__ inline GPlan gplan(const GDesc& d, int KW) {
   off = (off + 15) / 16 * 16;
   p.cfg = off; off += (size_t)d.G * d.NW * 8;
   p.bars = off; off += 64;
-  // MN-major A operands are read as M = 128 (64) rows = 16 (8) chunks from their
-  // start: the rows past the real ones are junk accumulator rows nobody reads,
-  // but the reads must stay inside the allocation
+  // MN-major A operands of the weight gradient (layers >= 1) are read as M = 64
+  // rows = 8 chunks from their start: the rows past the real ones are junk
+  // accumulator rows nobody reads, but the reads must stay inside the allocation
   const size_t last_a = p.sets + (size_t)(d.L - 3) * p.set_bytes;
-  const size_t span = (size_t)(d.wg_m64 ? 8 : 16) * d.rows_total * 16 + (size_t)d.rows_total * 16;
+  const size_t span = (size_t)8 * d.rows_total * 16 + (size_t)d.rows_total * 16;
   if (last_a + span > off) off = last_a + span;
   const size_t spin_span = (size_t)16 * d.GW * 16 + (size_t)d.rows_total * 16;
   if (p.spin + spin_span > off) off = p.spin + spin_span;
@@ -474,9 +473,10 @@ conv_grad_tc_kernel(GDesc d, const uint64_t* __restrict__ packed, const float* _
           colsum16_add(v, lane, my_slot + k * pl.slot_floats + l * kC);
         }
         sync_async();
-        // weight-gradient GEMMs, one accumulator of 32 columns per tap
+        // weight-gradient GEMMs, one accumulator of 32 columns per tap; M = 64 on the
+        // activation planes (half the A-operand fetch of M = 128), M = 128 on the spin plane
         const uint32_t hi_mn = plane_units | (1u << 14);          // MN-major: SBO = plane stride, LBO = 8 units
-        const uint32_t idesc_mn = (1u << 4) | ((uint32_t)((d.wg_m64 && l > 0) ? 4u : 8u) << 24) | (1u << 15) |
+        const uint32_t idesc_mn = (1u << 4) | ((uint32_t)(l > 0 ? 4u : 8u) << 24) | (1u << 15) |
                                   (1u << 16) | ((uint32_t)(kSlotCols >> 3) << 17);
         const uint32_t b_units = (smem_u32(wdset) >> 4) + (uint32_t)home_off;
         if (l == 0) {
@@ -526,13 +526,12 @@ conv_grad_tc_kernel(GDesc d, const uint64_t* __restrict__ packed, const float* _
             }
             commit_and_wait();
             // drain: accumulator row = (chunk_h, split_h, 8 ci), columns = (chunk_d, split_d, 8 co);
-            // d W[tap][ci][co] = D11 + (D12 + D21) / S + D22 / S^2.  M = 128: row m in lane m (warps
-            // with q = 0); M = 64: rows 16 i + r in lane 32 i + r (q = 0, 1).
-            const bool drains = d.wg_m64 ? (q < 2) : (q == 0);
-            if (drains) {
+            // d W[tap][ci][co] = D11 + (D12 + D21) / S + D22 / S^2.  M = 64: rows 16 i + r in
+            // lane 32 i + r (lane quarters q = 0, 1).
+            if (q < 2) {
               const int sh = (lane >> 3) & 1;
-              const int ci = (d.wg_m64 ? q * 8 : (lane >> 4) * 8) + (lane & 7);
-              const bool active = d.wg_m64 ? lane < 16 : true;
+              const int ci = q * 8 + (lane & 7);
+              const bool active = lane < 16;
               for (int tap = t0 + (warp >> 2); tap < t1; tap += 2) {   // two warps share a lane quarter
                 const uint32_t trow = tmem + ((uint32_t)(32 * q) << 16) + (uint32_t)((tap - t0) * kSlotCols);
                 uint32_t c0[16], c1[16];
@@ -667,10 +666,6 @@ bool make_gdesc(const cgsvmc_ansatz* a, int64_t B, GDesc* out) {
   d.n_tensor = d.L - 2;
   d.n_pairs = (d.kx + 1) / 2;
   d.wbuf_bytes = d.kx * d.ky * 3 * kC * kC * 2;
-  {
-    const char* e = getenv("CGSVMC_CONV_TC_GRAD_M64");
-    d.wg_m64 = e != nullptr && atoi(e) == 0 ? 0 : 1;   // default: M = 64 (half the A-operand fetch); 0 selects M = 128
-  }
   d.P = a->n_params;
   for (int l = 0; l < d.L; ++l) { d.w_off[l] = a->offsets[2 * l]; d.b_off[l] = a->offsets[2 * l + 1]; }
   // the largest batch that fits, but do not starve the grid

@@ -101,21 +101,16 @@ int launch_adam(float* params, float* m, float* v, int64_t n, const float* grad,
                 const double* stats, float inv_nb, float lr, const float* lr_dev, float b1, float b2,
                 float eps, uint64_t t, const uint64_t* t_dev, cudaStream_t s);
 
-// ---- pure RBM (num_layers == 0) fast path (rbm.cu) ----
+// ---- pure RBM (num_layers == 0): amplitudes, replay and large-bond local energy (rbm.cu) ----
 bool rbm_fast_supported(const cgsvmc_ansatz* a);
 int rbm_log_amp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, float* out,
                 cudaStream_t s);
-int rbm_mc_steps(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, int n_steps, uint64_t seed,
-                 uint64_t walker0, uint64_t step0, unsigned long long* accept_count,
-                 float* log_amp_out, cudaStream_t s);
 int rbm_mc_replay(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, const float* u_sites,
                   const float* u_acc, int32_t* down, int32_t* up, float* log_ratio,
                   uint8_t* accept, cudaStream_t s);
 int rbm_local_energy(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed,
                      int64_t B, float* e_loc, float* log_amp_out, float* diag_out,
                      float* off_out, cudaStream_t s);
-int rbm_grad(cgsvmc_ansatz* a, const uint64_t* packed, const float* weights, int64_t B, int K,
-             float* out, cudaStream_t s);
 
 // ---- pure RBM, second generation (rbm2.cu): ratio tables, 4 walkers per warp ----
 // h may be NULL in rbm2_supported (sampler only).

@@ -8,6 +8,12 @@
 // (SURVEY.md appendix A.2), so a Metropolis step or an off-diagonal matrix
 // element costs O(H) instead of the O(N H) forward pass the reference runs
 // twice per step (graph_builders.py:54-55, 74) / once per bond (operators.py:168).
+//
+// The sampler and the gradient sums of this ansatz run in rbm2 (rbm2.cu), which
+// plans every shape accepted here.  This file keeps what rbm2 does not cover:
+// the amplitudes (log_amp), the one-step replay of the reference's Metropolis
+// step (parity hook), and the local energy of Hamiltonians whose bond staging
+// does not fit rbm2's shared memory (N = 256, H = 144: rbm2 takes at most 200 bonds).
 #include "common.cuh"
 #include "internal.h"
 
@@ -141,68 +147,9 @@ rbm_log_amp_kernel(RbmParams p, const uint64_t* __restrict__ packed, int64_t B,
 }
 
 // ---------------------------------------------------------------------------
-// K2: persistent Metropolis sampler, graph_builders.py:54-89 x n_steps
+// K2 replay: one Metropolis step consuming caller-supplied uniforms
+// (graph_builders.py:59-79 verbatim)
 // ---------------------------------------------------------------------------
-template <int NW, int KJ, bool WS>
-__global__ void __launch_bounds__(kThreads)
-rbm_mc_kernel(RbmParams p, uint64_t* __restrict__ packed, int64_t B, int n_steps, uint64_t seed,
-              uint64_t walker0, uint64_t step0, unsigned long long* accept_count,
-              float* __restrict__ log_amp_out) {
-  extern __shared__ float smem[];
-  const float *a_s, *Wp; int ldw;
-  stage_params<KJ, WS>(p, smem, a_s, Wp, ldw);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  unsigned int n_acc = 0;
-  for (int64_t b = (int64_t)blockIdx.x * kWarps + warp; b < B; b += (int64_t)gridDim.x * kWarps) {
-    uint64_t s[NW], dnmask[NW]; float th[KJ], lc[KJ];
-    load_spins<NW>(packed, b, s);
-    init_theta<NW, KJ, WS>(p, Wp, ldw, s, lane, th, lc);
-    int n_up = 0;
-#pragma unroll
-    for (int w = 0; w < NW; ++w) n_up += __popcll(s[w]);
-    const int n_dn = p.N - n_up;
-    const bool can_move = n_up > 0 && n_dn > 0;
-    Philox4 rnd = {0, 0, 0, 0};
-    for (int step = 0; step < n_steps && can_move; ++step) {
-      if ((step & 31) == 0)   // lane l draws the block of step + l
-        rnd = walker_step_random(seed, walker0 + (uint64_t)b, step0 + (uint64_t)(step + lane));
-      const int src = step & 31;
-      const uint32_t r0 = __shfl_sync(CGSVMC_FULL_MASK, rnd.x, src);
-      const uint32_t r1 = __shfl_sync(CGSVMC_FULL_MASK, rnd.y, src);
-      const uint32_t r2 = __shfl_sync(CGSVMC_FULL_MASK, rnd.z, src);
-      // uniformly random up site and uniformly random down site
-      // (argmax / argmin of sigma * u, graph_builders.py:59-65)
-      const int k_up = __umulhi(r0, (uint32_t)n_up);
-      const int k_dn = __umulhi(r1, (uint32_t)n_dn);
-#pragma unroll
-      for (int w = 0; w < NW; ++w) dnmask[w] = ~s[w] & valid_mask_word(p.N, w);
-      const int up = select_kth_bit<NW>(s, k_up, lane);
-      const int dn = select_kth_bit<NW>(dnmask, k_dn, lane);
-      float tn[KJ], ln[KJ];
-      const float dl = exchange_log_ratio<KJ, WS>(p, a_s, Wp, ldw, up, dn, lane, th, lc, tn, ln);
-      // accept iff |psi'/psi| > sqrt(u)  <=>  exp(2 dl) > u   (strict; NaN rejects)
-      const float prob = fast_exp(2.f * dl);
-      if (prob > u32_to_unit(r2)) {
-#pragma unroll
-        for (int k = 0; k < KJ; ++k) { th[k] = tn[k]; lc[k] = ln[k]; }
-        flip_bit<NW>(s, up);
-        flip_bit<NW>(s, dn);
-        ++n_acc;
-      }
-    }
-    if (lane == 0) {
-#pragma unroll
-      for (int w = 0; w < NW; ++w) packed[b * NW + w] = s[w];
-    }
-    if (log_amp_out != nullptr) {
-      const float z = full_log_amp<NW, KJ>(p, a_s, s, lane, lc);
-      if (lane == 0) log_amp_out[b] = z;
-    }
-  }
-  if (accept_count != nullptr && lane == 0 && n_acc) atomicAdd(accept_count, (unsigned long long)n_acc);
-}
-
-// One step consuming caller-supplied uniforms (graph_builders.py:59-79 verbatim).
 template <int NW, int KJ, bool WS>
 __global__ void __launch_bounds__(kThreads)
 rbm_mc_replay_kernel(RbmParams p, uint64_t* __restrict__ packed, int64_t B,
@@ -306,108 +253,6 @@ rbm_local_energy_kernel(RbmParams p, const int2* __restrict__ bonds_ij,
 }
 
 // ---------------------------------------------------------------------------
-// K4: weighted sum of O_b = d z_b / d params (SURVEY.md appendix A.2/A.5):
-//   dz/da_i = sigma_i, dz/da0 = 1, dz/dW_ij = sigma_i tanh theta_j, dz/dc_j = tanh theta_j.
-// Every parameter is written as sign(i) * T[j] with an extra "ones" column
-// j = H and an extra all-ones spin word (i = -1), so one accumulation loop
-// serves the four tensors.
-// ---------------------------------------------------------------------------
-constexpr int kGradTile = 32;     // walkers per tile
-constexpr int kGradE = 16;        // parameter entries per thread
-
-template <int NW, int KJ, bool WS, int K>
-__global__ void __launch_bounds__(kThreads)
-rbm_grad_kernel(RbmParams p, const uint64_t* __restrict__ packed, const float* __restrict__ weights,
-                int64_t B, int64_t walkers_per_cta, int64_t P, float* __restrict__ partials) {
-  extern __shared__ float smem[];
-  const float *a_s, *Wp; int ldw;
-  const int param_floats = round_up(p.N, 32) + (WS ? p.N * 32 * KJ : 0);
-  const int HT = p.H + 1;
-  float* T_s = smem + round_up(param_floats, 4);                         // [tile][HT]
-  float* w_s = T_s + round_up(kGradTile * HT, 4);                        // [K][tile]
-  uint64_t* sp_s = reinterpret_cast<uint64_t*>(w_s + K * kGradTile);     // [tile][NW + 1]
-  stage_params<KJ, WS>(p, smem, a_s, Wp, ldw);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-
-  // decode this thread's parameter entries
-  int ej[kGradE], eword[kGradE], ebit[kGradE];
-  const int64_t e0 = (int64_t)blockIdx.y * (kThreads * kGradE) + threadIdx.x;
-  const int64_t w_begin = p.N + 1, w_end = w_begin + (int64_t)p.N * p.H;
-#pragma unroll
-  for (int m = 0; m < kGradE; ++m) {
-    const int64_t e = e0 + (int64_t)m * kThreads;
-    int i = -1, j = p.H;
-    if (e < p.N) { i = (int)e; }
-    else if (e == p.N) { }
-    else if (e < w_end) { const int q = (int)(e - w_begin); i = q / p.H; j = q - i * p.H; }
-    else if (e < P) { j = (int)(e - w_end); }
-    ej[m] = j;
-    eword[m] = i < 0 ? NW : (i >> 6);
-    ebit[m] = i < 0 ? 0 : (i & 63);
-  }
-  float acc[K][kGradE];
-#pragma unroll
-  for (int k = 0; k < K; ++k)
-#pragma unroll
-    for (int m = 0; m < kGradE; ++m) acc[k][m] = 0.f;
-
-  const int64_t b_begin = (int64_t)blockIdx.x * walkers_per_cta;
-  const int64_t b_end = min(B, b_begin + walkers_per_cta);
-  for (int64_t t0 = b_begin; t0 < b_end; t0 += kGradTile) {
-    // phase 1: tanh(theta) rows, spins and weights of the tile
-    for (int wb = warp; wb < kGradTile; wb += kWarps) {
-      const int64_t b = t0 + wb;
-      if (b < b_end) {
-        uint64_t s[NW]; float th[KJ], lc[KJ];
-        load_spins<NW>(packed, b, s);
-        init_theta<NW, KJ, WS>(p, Wp, ldw, s, lane, th, lc);
-#pragma unroll
-        for (int k = 0; k < KJ; ++k) {
-          const int j = lane + 32 * k;
-          if (j < p.H) T_s[wb * HT + j] = tanh_accurate(th[k]);
-        }
-        if (lane == 0) {
-          T_s[wb * HT + p.H] = 1.f;
-#pragma unroll
-          for (int w = 0; w < NW; ++w) sp_s[wb * (NW + 1) + w] = s[w];
-          sp_s[wb * (NW + 1) + NW] = ~0ull;
-        }
-        if (lane < K) w_s[lane * kGradTile + wb] = weights[(int64_t)lane * B + b];
-      } else {
-        for (int j = lane; j < HT; j += 32) T_s[wb * HT + j] = 0.f;
-        if (lane <= NW) sp_s[wb * (NW + 1) + lane] = ~0ull;
-        if (lane < K) w_s[lane * kGradTile + wb] = 0.f;
-      }
-    }
-    __syncthreads();
-    // phase 2: acc[k][entry] += w_k * sign_i * T_j
-    for (int wb = 0; wb < kGradTile; ++wb) {
-      float wk[K];
-#pragma unroll
-      for (int k = 0; k < K; ++k) wk[k] = w_s[k * kGradTile + wb];
-      const uint64_t* sp = sp_s + wb * (NW + 1);
-      const float* Trow = T_s + wb * HT;
-#pragma unroll
-      for (int m = 0; m < kGradE; ++m) {
-        const uint32_t flip = (uint32_t)(((sp[eword[m]] >> ebit[m]) & 1ull) ^ 1ull) << 31;
-        const float v = __uint_as_float(__float_as_uint(Trow[ej[m]]) ^ flip);
-#pragma unroll
-        for (int k = 0; k < K; ++k) acc[k][m] = fmaf(wk[k], v, acc[k][m]);
-      }
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int m = 0; m < kGradE; ++m) {
-    const int64_t e = e0 + (int64_t)m * kThreads;
-    if (e < P) {
-#pragma unroll
-      for (int k = 0; k < K; ++k) partials[((int64_t)blockIdx.x * K + k) * P + e] = acc[k][m];
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------
 // host-side dispatch
 // ---------------------------------------------------------------------------
 RbmParams make_params(const cgsvmc_ansatz* a) {
@@ -492,23 +337,6 @@ int rbm_log_amp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, float
   return cuda_fail(cudaGetLastError(), "rbm_log_amp launch");
 }
 
-int rbm_mc_steps(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, int n_steps, uint64_t seed,
-                 uint64_t walker0, uint64_t step0, unsigned long long* accept_count,
-                 float* log_amp_out, cudaStream_t st) {
-  const RbmParams p = make_params(a);
-  const Geometry g = geometry(a);
-  const int grid = grid_for(a, B);
-  const size_t smem = g.param_bytes;
-#define BODY(NWV, KJV, WSV)                                                        \
-  { auto kern = rbm_mc_kernel<NWV, KJV, WSV>;                                     \
-    if (int rc = set_smem(kern, smem)) return rc;                                 \
-    kern<<<grid, kThreads, smem, st>>>(p, packed, B, n_steps, seed, walker0, step0, \
-                                       accept_count, log_amp_out); }
-  RBM_DISPATCH(BODY)
-#undef BODY
-  return cuda_fail(cudaGetLastError(), "rbm_mc_steps launch");
-}
-
 int rbm_mc_replay(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, const float* u_sites,
                   const float* u_acc, int32_t* down, int32_t* up, float* log_ratio,
                   uint8_t* accept, cudaStream_t st) {
@@ -541,43 +369,6 @@ int rbm_local_energy(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t
   RBM_DISPATCH(BODY)
 #undef BODY
   return cuda_fail(cudaGetLastError(), "rbm_local_energy launch");
-}
-
-int rbm_grad(cgsvmc_ansatz* a, const uint64_t* packed, const float* weights, int64_t B, int K,
-             float* out, cudaStream_t st) {
-  const RbmParams p = make_params(a);
-  const Geometry g = geometry(a);
-  const int64_t P = a->n_params;
-  const int chunks = (int)((P + kThreads * kGradE - 1) / (kThreads * kGradE));
-  int64_t groups = std::max<int64_t>(1, (2 * (int64_t)a->num_sms) / chunks);
-  groups = std::min<int64_t>(groups, (B + kGradTile - 1) / kGradTile);
-  int64_t per_cta = (B + groups - 1) / groups;
-  per_cta = (per_cta + kGradTile - 1) / kGradTile * kGradTile;
-  groups = (B + per_cta - 1) / per_cta;
-  if (int rc = ensure_scratch(a, (size_t)groups * 2 * P * sizeof(float))) return rc;
-  const int nw = pick_nw(a->desc.n_sites);
-  dim3 grid((unsigned)groups, (unsigned)chunks);
-  // kernels take one or two weight columns; more columns are processed in pairs
-  for (int k0 = 0; k0 < K; k0 += 2) {
-    const int kk = std::min(2, K - k0);
-    const float* w = weights + (int64_t)k0 * B;
-    const size_t smem = round_up((int)g.param_bytes, 16) +
-                        (size_t)round_up(kGradTile * (p.H + 1), 4) * 4 + (size_t)kk * kGradTile * 4 +
-                        (size_t)kGradTile * (nw + 1) * 8 + 16;
-#define BODY_K(NWV, KJV, WSV, KV)                                                  \
-  { auto kern = rbm_grad_kernel<NWV, KJV, WSV, KV>;                               \
-    if (int rc = set_smem(kern, smem)) return rc;                                 \
-    kern<<<grid, kThreads, smem, st>>>(p, packed, w, B, per_cta, P, a->scratch); }
-#define BODY(NWV, KJV, WSV)                                                        \
-  if (kk == 1) BODY_K(NWV, KJV, WSV, 1) else BODY_K(NWV, KJV, WSV, 2)
-    RBM_DISPATCH(BODY)
-#undef BODY
-#undef BODY_K
-    if (int rc = cuda_fail(cudaGetLastError(), "rbm_grad launch")) return rc;
-    if (int rc = launch_reduce_partials(a->scratch, (int)groups, (int64_t)kk * P,
-                                        out + (int64_t)k0 * P, st)) return rc;
-  }
-  return CGSVMC_OK;
 }
 
 }  // namespace cgsvmc

@@ -173,12 +173,8 @@ bool base_plan(const cgsvmc_ansatz* a, int64_t B, Plan* pl, bool walker) {
   pl->kjv = HP / 32;
   // 8 lanes per walker (four walkers per warp) while the state fits 128
   // registers, else 16; measured on B200 at C2: 8 lanes 100 us / step, 16 lanes
-  // 110 us (profiles/r01e_*).  CGSVMC_RBM2_LPW=16 forces the 16-lane layout.
-  static const int forced_lpw = [] {
-    const char* e = getenv("CGSVMC_RBM2_LPW");
-    return e != nullptr ? atoi(e) : 0;
-  }();
-  pl->lpw = (forced_lpw != 16 && pl->kjv <= 5) ? 8 : 16;
+  // 110 us (profiles/r01e_*).
+  pl->lpw = pl->kjv <= 5 ? 8 : 16;
   pl->im = make_image(d.n_sites, H, HP);
   pl->nw = n_words(d.n_sites) == 3 ? 4 : n_words(d.n_sites);
   const int wpw = 32 / pl->lpw, slots = variant_slots(pl->lpw, pl->kjv, walker);
@@ -284,11 +280,10 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
   pl.ws = walker_smem_bytes(pl.im, slots, true, do_eloc, nb, do_grad, mc) <= (size_t)a->max_smem_optin;
   // bond-pair table: 8 lanes per walker, at least one bond, pair index below 2^15,
   // and everything (image from F on + pair table + staging) in shared memory
-  static const bool pt_off = getenv("CGSVMC_RBM2_NO_PAIR_TABLE") != nullptr;
-  pl.pt = !pt_off && do_eloc && pl.ws && pl.lpw == 8 && nb >= 1 && nb < 16384 &&
+  pl.pt = do_eloc && pl.ws && pl.lpw == 8 && nb >= 1 && nb < 16384 &&
           walker_smem_bytes(pl.im, slots, true, do_eloc, nb, do_grad, mc, true) <= (size_t)a->max_smem_optin;
   // tables in global memory: the pair table too (read through L1 / L2)
-  const bool pt_global = !pt_off && do_eloc && !pl.ws && nb >= 1 && nb < 16384;
+  const bool pt_global = do_eloc && !pl.ws && nb >= 1 && nb < 16384;
   cgsvmc_ansatz::PairTable* slot =
       (pl.pt || pt_global) ? pair_slot(a, h, (size_t)2 * nb * pl.im.HP * 4) : nullptr;
   if (slot == nullptr) pl.pt = false;
@@ -325,9 +320,6 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
     const int np4 = round_up(pl.im.N + 1, 4), np8 = round_up(pl.im.N + 1, 8);
     A.tc_grad = (!off && pl.pt && do_grad && weights == nullptr && np8 == np4 && 3 * np8 <= 128 &&
                  pl.im.H < pl.im.HP && 3 * pl.im.HP <= 512 && (slots == 64 || slots == 128)) ? 1 : 0;
-    if (A.tc_grad && e != nullptr && atoi(e) == 2) A.tc_grad = 2;      // development: E_loc centred per segment
-    const char* sg = getenv("CGSVMC_RBM2_TC_SEGMENT");
-    A.tc_segment = sg != nullptr && atoi(sg) > 0 ? atoi(sg) : 8;
   }
   if (mc) A.configs_f32 = sweep->configs_f32;
   const int n_iters = mc && sweep->n_iters > 1 ? sweep->n_iters : 1;
@@ -362,9 +354,7 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
   uint64_t* const step_counter = mc ? sweep->advance_counter : nullptr;
   double* const snapshot = mc ? sweep->stats_snapshot : nullptr;
   if (fuse) {
-    // 2 = plain launch (development comparison: the spin wait then relies on
-    // the grid being co-resident because nothing else runs on the device)
-    A.fuse_reduce = (fuse_env != nullptr && atoi(fuse_env) == 2) ? 2 : 1;
+    A.fuse_reduce = 1;
     A.sync = a->grid_sync;
     A.out = out; A.n_out = (int64_t)K * P; A.stats = stats;
     A.counter = step_counter; A.advance = mc ? (uint64_t)sweep->n_steps * (uint64_t)n_iters : 0ull;

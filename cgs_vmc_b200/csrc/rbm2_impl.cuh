@@ -739,7 +739,7 @@ mc_kernel(Image im, const float* __restrict__ img_g, uint64_t* __restrict__ pack
 // would otherwise be paid in instruction fetches.
 template <int THREADS, int NCOL>
 __device__ __noinline__ void tcg_drain(uint32_t tmem, float* stg, int n_groups, float* part, int64_t P, int N, int H,
-                                       int NC, float e_center, bool add) {
+                                       int NC, bool add) {
   constexpr int LD = 20;                     // staging row stride (floats): 16-byte aligned rows
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int NPC = 8 * NC;
@@ -802,8 +802,7 @@ __device__ __noinline__ void tcg_drain(uint32_t tmem, float* stg, int n_groups, 
                     a3[4] = {p3.x, p3.y, p3.z, p3.w};
 #pragma unroll
         for (int u = 0; u < 4; ++u)
-          v[u] = fmaf(e_center, v[u],
-                      fmaf(fmaf(a3[u], 1.f / 2048.f, a2[u]), 1.f / 2048.f, a1[u]) * (1.f / kTcgPrescale));
+          v[u] = fmaf(fmaf(a3[u], 1.f / 2048.f, a2[u]), 1.f / 2048.f, a1[u]) * (1.f / kTcgPrescale);
       }
       float* row_w = part + (size_t)k * P + (size_t)(N + 1) + (size_t)i * H;    // W[i][.] (i < N), c[.] (i == N)
 #pragma unroll
@@ -860,7 +859,6 @@ struct WalkerArgs {
   // TMEM for the whole launch) instead of the FP32 register tiles; planned by
   // the host when the shapes fit (N <= 39, H <= 159: the C2 class)
   int tc_grad;
-  int tc_segment;   // passes accumulated in TMEM between two drains (truncating fp32 accumulation)
   // walkers given as the reference's float32 [B][N] of +-1 instead of packed
   // words (the packed configurations are still written to packed_rw)
   const float* configs_f32;
@@ -1056,19 +1054,16 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
   //   drained once.
   constexpr int NCOL = HP;                       // B columns: H real ones + the constant 1 (needs H < HP)
   constexpr int NB = NCOL / 8;                   // B chunks per split
-  const bool tcg = PT && A.do_grad && A.tc_grad;
+  // (planned only for N <= 39: one spin word, so the wider kernels carry no tensor-core code)
+  const bool tcg = PT && NW == 1 && A.do_grad && A.tc_grad;
   const int NC = (im.N + 1 + 7) / 8;             // A chunks per group
   uint32_t tmem = 0;
   // The tensor cores accumulate in fp32 with truncation: over the 200 MMA steps
   // of a 50-iteration launch the coherent sum E sum_b O_b drifted by 1.3e-5 of
-  // its value.  The accumulators are therefore drained every A.tc_segment
+  // its value.  The accumulators are therefore drained every kTcgSegment
   // passes (1.7e-6 against the FP32 register tiles after 50 iterations,
-  // profiles/r02u_precision.txt).  Development option (A.tc_grad == 2): the
-  // weight planes hold E_loc - e_center, e_center = mean local energy of the
-  // CTA's walkers in the first pass of the segment, S_1 += sum_b (E_b -
-  // e_center) O_b + e_center S_0 in the drain -- better for equilibrated
-  // walkers, worse while the energy still drifts; off by default.
-  float e_center = 0.f;
+  // profiles/r02u_precision.txt).
+  constexpr int kTcgSegment = 8;
   // drain: T_s and ws_s (contiguous, free between two passes) stage up to four
   // 16-column chunks at a time, one per group of four warps
   const int drain_groups = max(1, min(min(THREADS / 128, 4),
@@ -1192,11 +1187,9 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
       }
     }
     // the MMAs of the previous pass have read the operand planes; a full
-    // segment of A.tc_segment passes is drained before the next one starts
-    // (bounds the truncating accumulation in TMEM and lets e_center follow
-    // the energy of the walkers)
-    const bool seg_start = tcg && (batch_no % A.tc_segment) == 0;
-    const bool centre = seg_start && A.tc_grad == 2;          // development: E_loc centred per segment
+    // segment of kTcgSegment passes is drained before the next one starts
+    // (bounds the truncating accumulation in TMEM)
+    const bool seg_start = tcg && (batch_no % kTcgSegment) == 0;
     if (tcg && batch_no > 0) {
       const uint32_t bar_a = smem_u32(mma_bar), parity = (uint32_t)(batch_no - 1) & 1u;
       uint32_t ok = 0;
@@ -1204,7 +1197,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
         asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
                      : "=r"(ok) : "r"(bar_a), "r"(parity) : "memory");
       if (seg_start) {
-        tcg_drain<THREADS, NCOL>(tmem, T_s, drain_groups, part, A.P, im.N, im.H, NC, e_center, n_drained > 0);
+        tcg_drain<THREADS, NCOL>(tmem, T_s, drain_groups, part, A.P, im.N, im.H, NC, n_drained > 0);
         ++n_drained;
         // the staging went through the operand planes: rows of empty slots must read as zero again
         for (int e = threadIdx.x; e < SLOTS * HP / 4; e += THREADS)
@@ -1271,19 +1264,6 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
           if (A.off) A.off[ob] = off;
         }
       }
-      if (centre) {
-        // e_center: every thread sums the staged local energies in the same order
-        if (valid && sub == 0) e_s[slot] = e_val;
-      }
-    }
-    if (centre) {
-      __syncthreads();
-      float acc_e = 0.f;
-      for (int sb = 0; sb < n_valid; ++sb) acc_e += e_s[sb];
-      acc_e /= (float)n_valid;
-      e_center = fabsf(acc_e) < 1.0e30f ? acc_e : 0.f;       // (NaN / inf: no centring)
-    }
-    if (warp_on) {
       if (A.do_grad && valid) {
         // stage tanh(theta) = p - m, the signed weights w_k sigma_i and E_loc
         float w0, w1;
@@ -1323,7 +1303,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
           // A planes: sigma, then the three fp16 pieces of w1 sigma 2^-20 (w0 = 1 on this path):
           // x = x1 + x2 / S + x3 / S^2, 33 mantissa bits; the prescale keeps |E_loc| < 6.8e10
           // inside the fp16 range, small values stay exact through the scaled residuals
-          float rem = (w1 - e_center) * kTcgPrescale;
+          float rem = w1 * kTcgPrescale;
           uint32_t piece[3];
 #pragma unroll
           for (int g = 0; g < 3; ++g) {
@@ -1396,7 +1376,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
         asm volatile("{ .reg .pred p; elect.sync _|p, 0xffffffff; selp.u32 %0, 1, 0, p; }" : "=r"(elected));
         if (elected) {
           for (int ks = 0; ks < SLOTS / 16; ++ks) {
-            const uint32_t accf = ((batch_no % A.tc_segment) > 0 || ks > 0) ? 1u : 0u;
+            const uint32_t accf = ((batch_no % kTcgSegment) > 0 || ks > 0) ? 1u : 0u;
             const uint64_t a0d = ((uint64_t)hi << 32) | ((a_units + (uint32_t)(16 * ks)) | (8u << 16));
             const uint64_t a3d = ((uint64_t)hi << 32) | ((a_units + (uint32_t)(3 * NC * SLOTS + 16 * ks)) | (8u << 16));
             const uint64_t b1d = ((uint64_t)hi << 32) | ((b_units + (uint32_t)(16 * ks)) | (8u << 16));
@@ -1550,7 +1530,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
     while (!ok)
       asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
                    : "=r"(ok) : "r"(bar_a), "r"(parity) : "memory");
-    tcg_drain<THREADS, NCOL>(tmem, T_s, drain_groups, part, A.P, im.N, im.H, NC, e_center, n_drained > 0);
+    tcg_drain<THREADS, NCOL>(tmem, T_s, drain_groups, part, A.P, im.N, im.H, NC, n_drained > 0);
   }
   if (A.do_grad) {
 #pragma unroll
@@ -1617,7 +1597,7 @@ int launch_walker_variant(const Plan& pl, const float* img, const WalkerArgs& A,
   do {                                                                            \
     auto kern = walker_kernel<NW, LPW, KJV, WSV, MCV, PTV>;                       \
     if (int rc = opt_in_smem(kern, pl.walker_smem)) return rc;                    \
-    if (A.fuse_reduce == 1) {                                                     \
+    if (A.fuse_reduce) {                                                          \
       cudaLaunchConfig_t cfg = {};                                                \
       cfg.gridDim = dim3(pl.grid); cfg.blockDim = dim3(THREADS);                  \
       cfg.dynamicSmemBytes = pl.walker_smem; cfg.stream = st;                     \
@@ -1651,11 +1631,6 @@ inline int variant_slots(int lpw, int kjv, bool walker) {
     case 8 * 16 + 3: return CALL(NWV, 8, 3);                 \
     case 8 * 16 + 4: return CALL(NWV, 8, 4);                 \
     case 8 * 16 + 5: return CALL(NWV, 8, 5);                 \
-    case 16 * 16 + 1: return CALL(NWV, 16, 1);               \
-    case 16 * 16 + 2: return CALL(NWV, 16, 2);               \
-    case 16 * 16 + 3: return CALL(NWV, 16, 3);               \
-    case 16 * 16 + 4: return CALL(NWV, 16, 4);               \
-    case 16 * 16 + 5: return CALL(NWV, 16, 5);               \
     case 16 * 16 + 6: return CALL(NWV, 16, 6);               \
     case 16 * 16 + 7: return CALL(NWV, 16, 7);               \
     case 16 * 16 + 8: return CALL(NWV, 16, 8);               \

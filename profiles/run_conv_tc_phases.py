@@ -3,7 +3,7 @@
 barrier) against epilogue, per tensor layer, from the counters of the timing
 build (`python __graft_entry__.py --timing` -> libcgsvmc_timing.so).
 
-  CGSVMC_LIBRARY=cgs_vmc_b200/libcgsvmc_timing.so python profiles/run_conv_tc_phases.py [--ctas 1|2]
+  CGSVMC_LIBRARY=cgs_vmc_b200/libcgsvmc_timing.so python profiles/run_conv_tc_phases.py
 """
 import argparse
 import ctypes
@@ -17,10 +17,8 @@ sys.path.insert(0, REPO)
 
 def main():
   ap = argparse.ArgumentParser()
-  ap.add_argument('--ctas', default='2')
   ap.add_argument('--walkers', type=int, default=8192)
   args = ap.parse_args()
-  os.environ['CGSVMC_CONV_TC_CTAS'] = args.ctas
   os.environ.setdefault('CGSVMC_LIBRARY', os.path.join(REPO, 'cgs_vmc_b200', 'libcgsvmc_timing.so'))
   import numpy as np
   import torch
@@ -44,7 +42,7 @@ def main():
     torch.cuda.synchronize()
     lib.cgsvmc_debug_conv_tc_phases(out)
     mma, epi, layers, fwd = [int(v) for v in out]
-    print(json.dumps({'kernel': name, 'ctas_per_sm': int(args.ctas), 'ms': e0.elapsed_time(e1),
+    print(json.dumps({'kernel': name, 'ms': e0.elapsed_time(e1),
                       'tensor_layers': layers, 'forwards': fwd,
                       'mma_phase_cycles_per_layer': mma / max(1, layers),
                       'epilogue_cycles_per_layer': epi / max(1, layers),
