@@ -32,7 +32,7 @@ EXPORTS = [
     'cgsvmc_propose_exchange', 'cgsvmc_accept_exchange', 'cgsvmc_local_energy_from_amps',
     'cgsvmc_swo_weights', 'cgsvmc_adam_step', 'cgsvmc_batch_step_fed', 'cgsvmc_batch_steps',
     'cgsvmc_epoch_end', 'cgsvmc_pack_configs_host', 'cgsvmc_upload_configs',
-    'cgsvmc_conv_periodic',
+    'cgsvmc_conv_periodic', 'cgsvmc_log_amp_jvp',
 ]
 
 
@@ -81,6 +81,7 @@ def load():
   lib.cgsvmc_flip_enum.argtypes = [vp, vp, i64, vp, vp, vp]
   lib.cgsvmc_local_energy.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, vp]
   lib.cgsvmc_weighted_grad_sum.argtypes = [vp, vp, vp, i64, i32, vp, vp]
+  lib.cgsvmc_log_amp_jvp.argtypes = [vp, vp, i64, vp, vp, vp]
   lib.cgsvmc_energy_stats.argtypes = [vp, i64, vp, vp]
   lib.cgsvmc_accumulate.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, vp]
   lib.cgsvmc_batch_step.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, i32, u64, u64, u64, vp, vp, vp]
@@ -277,6 +278,21 @@ class Ansatz:
                                           b, k, _ptr(out), _stream()))
     return out
 
+  def log_amp_jvp(self, packed, tangent, out=None):
+    """out[b] = sum_p d z_b / d params_p * tangent[p] (float32 [B]) for a
+    tangent in the flat parameter layout: the forward counterpart of
+    weighted_grad_sum (cgsvmc_log_amp_jvp; pure RBM only, NotImplementedError
+    otherwise)."""
+    self._sync_params()
+    b = packed.shape[0]
+    _want(packed, torch.int64, (b, n_words(self.n_sites)), 'packed')
+    _want(tangent, torch.float32, (self.num_params,), 'tangent')
+    if out is None:
+      out = torch.empty(b, dtype=torch.float32, device=packed.device)
+    else:
+      _want(out, torch.float32, (b,), 'out')
+    check(load().cgsvmc_log_amp_jvp(self._handle, _ptr(packed), b, _ptr(tangent), _ptr(out), _stream()))
+    return out
 
   def accumulate(self, ham, packed, sums, stats, e_loc_out=None, log_amp_out=None):
     """One session.run(accumulate_gradients) (training.py:539-558): sums [2, P]

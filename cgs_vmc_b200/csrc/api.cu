@@ -423,6 +423,22 @@ int cgsvmc_weighted_grad_sum(const cgsvmc_ansatz* a, const uint64_t* packed, con
   return net_grad(am, packed, weights, B, K, out, (cudaStream_t)stream);
 }
 
+int cgsvmc_log_amp_jvp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, const float* tangent,
+                       float* jvp_out, void* stream) {
+  NvtxRange range("cgsvmc:K1 log_amp_jvp");
+  if (int rc = check_ready(a)) return rc;
+  if (B < 0) return invalid("log_amp_jvp: n_walkers < 0");
+  // before the empty-batch return, so that a call with no walkers probes for support
+  if (!rbm_fast_supported(a)) {
+    set_error("log_amp_jvp: built for the pure RBM only (rbm, no hidden layers, H <= 256, "
+              "1, 2 or 4 spin words)");
+    return CGSVMC_ERR_UNSUPPORTED;
+  }
+  if (B == 0) return CGSVMC_OK;
+  if (packed == nullptr || tangent == nullptr || jvp_out == nullptr) return invalid("log_amp_jvp: NULL buffer");
+  return rbm_log_amp_jvp(a, packed, B, tangent, jvp_out, (cudaStream_t)stream);
+}
+
 int cgsvmc_accumulate(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, int64_t B,
                       float* e_loc_out, float* log_amp_out, float* sums, double* stats, void* stream) {
   NvtxRange range("cgsvmc:K3+K4+K5 accumulate");

@@ -101,10 +101,14 @@ int launch_adam(float* params, float* m, float* v, int64_t n, const float* grad,
                 const double* stats, float inv_nb, float lr, const float* lr_dev, float b1, float b2,
                 float eps, uint64_t t, const uint64_t* t_dev, cudaStream_t s);
 
-// ---- pure RBM (num_layers == 0): amplitudes, replay and large-bond local energy (rbm.cu) ----
+// ---- pure RBM (num_layers == 0): amplitudes, their directional derivative, replay and
+//      large-bond local energy (rbm.cu) ----
 bool rbm_fast_supported(const cgsvmc_ansatz* a);
 int rbm_log_amp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, float* out,
                 cudaStream_t s);
+// out[b] = sum_p (d z_b / d params_p) tangent[p]   (tangent: device float [P], flat layout)
+int rbm_log_amp_jvp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, const float* tangent,
+                    float* out, cudaStream_t s);
 int rbm_mc_replay(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, const float* u_sites,
                   const float* u_acc, int32_t* down, int32_t* up, float* log_ratio,
                   uint8_t* accept, cudaStream_t s);

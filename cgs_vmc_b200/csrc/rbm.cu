@@ -11,7 +11,8 @@
 //
 // The sampler and the gradient sums of this ansatz run in rbm2 (rbm2.cu), which
 // plans every shape accepted here.  This file keeps what rbm2 does not cover:
-// the amplitudes (log_amp), the one-step replay of the reference's Metropolis
+// the amplitudes (log_amp) and their directional derivative (log_amp_jvp, the
+// forward half of the matrix-free S v of stochastic reconfiguration), the one-step replay of the reference's Metropolis
 // step (parity hook), and the local energy of Hamiltonians whose bond staging
 // does not fit rbm2's shared memory (N = 256, H = 144: rbm2 takes at most 200 bonds).
 #include "common.cuh"
@@ -147,6 +148,60 @@ rbm_log_amp_kernel(RbmParams p, const uint64_t* __restrict__ packed, int64_t B,
 }
 
 // ---------------------------------------------------------------------------
+// K1 tangent: y_b = sum_p (d z_b / d params_p) v_p for a tangent v in the flat
+// layout (v_a, v_a0, V, v_c), seen through `t` like the parameters through `p`:
+//   y = sum_j tanh(theta_j) u_j + v_a . sigma + v_a0,  u = V^T sigma + v_c.
+// theta and u are built in the same pass over the spin bits; W and V are
+// staged side by side when both fit (rbm_log_amp_jvp decides).  FP32 with a
+// fixed summation order: the result does not change from run to run.
+// ---------------------------------------------------------------------------
+template <int NW, int KJ, bool WS>
+__global__ void __launch_bounds__(kThreads)
+rbm_log_amp_jvp_kernel(RbmParams p, RbmParams t, const uint64_t* __restrict__ packed, int64_t B,
+                       float* __restrict__ out) {
+  extern __shared__ float smem[];
+  const float *a_s, *Wp, *va_s, *Vp; int ldw;
+  const int param_floats = round_up(p.N, 32) + (WS ? p.N * 32 * KJ : 0);
+  stage_params<KJ, WS>(p, smem, a_s, Wp, ldw);
+  stage_params<KJ, WS>(t, smem + param_floats, va_s, Vp, ldw);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int64_t b = (int64_t)blockIdx.x * kWarps + warp; b < B; b += (int64_t)gridDim.x * kWarps) {
+    uint64_t s[NW]; float th[KJ], u[KJ];
+    load_spins<NW>(packed, b, s);
+#pragma unroll
+    for (int k = 0; k < KJ; ++k) {
+      const int j = lane + 32 * k;
+      th[k] = j < p.H ? p.c[j] : 0.f;
+      u[k] = j < p.H ? t.c[j] : 0.f;
+    }
+#pragma unroll
+    for (int w = 0; w < NW; ++w) {
+      const int n_here = min(64, p.N - 64 * w);
+      const uint64_t word = s[w];
+      for (int bpos = 0; bpos < n_here; ++bpos) {
+        const uint32_t flip = (uint32_t)(((word >> bpos) & 1ull) ^ 1ull) << 31;
+        const float* wrow = Wp + (size_t)(64 * w + bpos) * ldw;
+        const float* vrow = Vp + (size_t)(64 * w + bpos) * ldw;
+#pragma unroll
+        for (int k = 0; k < KJ; ++k) {
+          const int j = lane + 32 * k;
+          if (WS || j < p.H) {
+            th[k] += __uint_as_float(__float_as_uint(wrow[j]) ^ flip);
+            u[k] += __uint_as_float(__float_as_uint(vrow[j]) ^ flip);
+          }
+        }
+      }
+    }
+    float part = 0.f;
+#pragma unroll
+    for (int k = 0; k < KJ; ++k) part = fmaf(tanhf(th[k]), u[k], part);
+    for (int i = lane; i < p.N; i += 32) part += get_bit<NW>(s, i) ? va_s[i] : -va_s[i];
+    const float y = warp_sum(part) + t.a0[0];
+    if (lane == 0) out[b] = y;
+  }
+}
+
+// ---------------------------------------------------------------------------
 // K2 replay: one Metropolis step consuming caller-supplied uniforms
 // (graph_builders.py:59-79 verbatim)
 // ---------------------------------------------------------------------------
@@ -255,16 +310,19 @@ rbm_local_energy_kernel(RbmParams p, const int2* __restrict__ bonds_ij,
 // ---------------------------------------------------------------------------
 // host-side dispatch
 // ---------------------------------------------------------------------------
-RbmParams make_params(const cgsvmc_ansatz* a) {
+// `flat` is a vector in the flat parameter layout: the parameters or a tangent.
+RbmParams make_params(const cgsvmc_ansatz* a, const float* flat) {
   RbmParams p;
   p.N = a->desc.n_sites;
   p.H = a->desc.layer_size;
-  p.a = a->params + a->offsets[0];
-  p.a0 = a->params + a->offsets[1];
-  p.W = a->params + a->offsets[2];
-  p.c = a->params + a->offsets[3];
+  p.a = flat + a->offsets[0];
+  p.a0 = flat + a->offsets[1];
+  p.W = flat + a->offsets[2];
+  p.c = flat + a->offsets[3];
   return p;
 }
+
+RbmParams make_params(const cgsvmc_ansatz* a) { return make_params(a, a->params); }
 
 int pick_kj(int H) { return H <= 64 ? 2 : H <= 128 ? 4 : H <= 160 ? 5 : 8; }
 int pick_nw(int N) { return n_words(N); }
@@ -335,6 +393,26 @@ int rbm_log_amp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, float
   RBM_DISPATCH(BODY)
 #undef BODY
   return cuda_fail(cudaGetLastError(), "rbm_log_amp launch");
+}
+
+int rbm_log_amp_jvp(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t B, const float* tangent,
+                    float* out, cudaStream_t st) {
+  const RbmParams p = make_params(a);
+  const RbmParams t = make_params(a, tangent);
+  // two parameter images (params, tangent) under the budget one has in geometry()
+  Geometry g = geometry(a);
+  const size_t base = (size_t)round_up(a->desc.n_sites, 32) * 4;
+  const size_t wbytes = (size_t)a->desc.n_sites * 32 * g.kj * 4;
+  g.ws = 2 * (base + wbytes) <= 96 * 1024;
+  const size_t smem = 2 * (base + (g.ws ? wbytes : 0));
+  const int grid = grid_for(a, B);
+#define BODY(NWV, KJV, WSV)                                                        \
+  { auto kern = rbm_log_amp_jvp_kernel<NWV, KJV, WSV>;                            \
+    if (int rc = set_smem(kern, smem)) return rc;                                 \
+    kern<<<grid, kThreads, smem, st>>>(p, t, packed, B, out); }
+  RBM_DISPATCH(BODY)
+#undef BODY
+  return cuda_fail(cudaGetLastError(), "rbm_log_amp_jvp launch");
 }
 
 int rbm_mc_replay(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, const float* u_sites,

@@ -8,6 +8,10 @@ different weight columns (SURVEY.md appendix A.5).  The Metropolis loops of the
 reference (one session.run per step) collapse into one persistent-kernel
 launch per sweep group; `session.run(train_ops.mc_step)` still performs a
 single step for drop-in callers.
+
+StochasticReconfigurationOptimizer goes beyond the reference: the natural
+gradient of VMC for the pure RBM, with S applied matrix-free through
+cgsvmc_log_amp_jvp and cgsvmc_weighted_grad_sum.
 """
 import collections
 import copy
@@ -387,6 +391,197 @@ class EnergyGradientOptimizer(WavefunctionOptimizer):
       session.run(train_ops.apply_gradients)
       energy = session.run(train_ops.metrics)
       session.run(train_ops.reset_gradients)
+    session.run(train_ops.epoch_increment)
+    return energy
+
+
+def sr_matvec(ansatz, packed, o_mean, v, n_samples, diag_shift, allreduce=distributed.allreduce_):
+  """(S + diag_shift I) v with S = <O O^T> - <O><O>^T over `n_samples` walkers,
+  without forming S: y_b = O_b . v - <O> . v over the local walkers `packed`
+  (one cgsvmc_log_amp_jvp launch), then sum_b y_b O_b (one
+  cgsvmc_weighted_grad_sum launch), summed over the walker shards by
+  `allreduce` (a float64 P-vector in, the sum over all shards out).  o_mean, v:
+  float64 [P] on the device; returns float64 [P]."""
+  y = ansatz.log_amp_jvp(packed, v.float())
+  y = (y.double() - torch.dot(o_mean, v)).float()
+  sv = ansatz.weighted_grad_sum(packed, y.reshape(1, -1))[0].double()
+  return allreduce(sv) / n_samples + diag_shift * v
+
+
+def conjugate_gradient(matvec, b, tolerance, max_iterations, check_every=5):
+  """Solves A x = b for a symmetric positive definite A given as `matvec`,
+  from x = 0, on b's device and dtype.  Stops once ||r|| <= tolerance ||b||,
+  tested every `check_every` iterations (each test is one device-to-host
+  read), or after `max_iterations`.  Returns (x, iterations, ||r|| / ||b||)
+  with r the recursively updated residual."""
+  x = torch.zeros_like(b)
+  b_norm = float(torch.linalg.vector_norm(b))
+  if b_norm == 0.0:
+    return x, 0, 0.0
+  tiny = torch.finfo(b.dtype).tiny
+  r = b.clone()
+  p = r.clone()
+  rs = torch.dot(r, r)
+  it = 0
+  while it < max_iterations:
+    ap = matvec(p)
+    alpha = rs / torch.dot(p, ap).clamp_min(tiny)
+    x.add_(alpha * p)
+    r.sub_(alpha * ap)
+    rs_new = torch.dot(r, r)
+    it += 1
+    if it % check_every == 0 and math.sqrt(float(rs_new)) <= tolerance * b_norm:
+      rs = rs_new
+      break
+    p = r + (rs_new / rs.clamp_min(tiny)) * p
+    rs = rs_new
+  return x, it, math.sqrt(float(rs)) / b_norm
+
+
+def _require_pure_rbm(wavefunction, n_sites):
+  """Stochastic reconfiguration needs cgsvmc_log_amp_jvp, which is built for the
+  pure RBM; checked before anything is allocated."""
+  ok = (isinstance(wavefunction, wavefunctions.RestrictedBoltzmannNetwork) and
+        wavefunction._num_layers == 0 and wavefunction._layer_size <= 256 and
+        n_sites <= 256 and _native.n_words(n_sites) != 3)
+  if not ok:
+    raise NotImplementedError(
+        'StochasticReconfiguration needs a single pure RBM: wavefunction_type=rbm with '
+        'num_fc_layers=0, fc_layer_size <= 256 and num_sites <= 128 or 193..256 (got %s, num_sites=%d)'
+        % (type(wavefunction).__name__, n_sites))
+
+
+class StochasticReconfigurationOptimizer(WavefunctionOptimizer):
+  """Stochastic reconfiguration (the natural gradient of VMC) for the pure RBM;
+  the reference has no such optimizer.
+
+  An epoch samples like EnergyGradientOptimizer.run_optimization_epoch (one
+  captured cgsvmc_batch_step per batch) and keeps the configurations every
+  batch is accumulated on.  With M the number of walkers of the epoch on all
+  ranks, <.> the mean over them and O_b = d log psi_b / d params, it then
+  solves
+    (S + sr_diag_shift I) delta = F,
+    S = <O O^T> - <O><O>^T,  F = <E O> - <E><O>
+  by conjugate gradient (float64 vectors, x0 = 0, ||r|| <= sr_cg_tolerance ||F||
+  or sr_cg_max_iterations), with S applied matrix-free (sr_matvec).  S and F
+  are the textbook covariances, WITHOUT the factor B that
+  EnergyGradientOptimizer's gradient carries.
+
+  delta goes through hparams.optimizer: optimizer=gradient is classic SR,
+  params -= lr delta, and is the recommended setting; with adam, Adam receives
+  delta as its gradient.  After every solve `cg_iterations`, `cg_residual`
+  (relative) and `direction` (delta) hold its result."""
+
+  def build_opt_ops(self, wavefunction, hamiltonian, hparams, shared_resources):
+    n_sites = hparams.num_sites
+    _require_pure_rbm(wavefunction, n_sites)
+    local_batch, walker_id0 = distributed.shard(hparams.batch_size)
+    configs = graph_builders.get_configs(shared_resources, local_batch, n_sites,
+                                         walker_id0=walker_id0)
+    mc_step, acc_rate = graph_builders.get_monte_carlo_sampling(
+        shared_resources, configs, wavefunction)
+    model = _Model(wavefunction, n_sites, hparams)
+    ansatz = model.ansatz
+    ham = hamiltonian.native(n_sites)
+    sums = engine.EnergyGradientSums(ansatz, local_batch)
+    if distributed.world_size() > 1:
+      total = types.SimpleNamespace(sums=torch.zeros_like(sums.sums),
+                                    stats=torch.zeros_like(sums.stats))
+    else:
+      total = sums
+    # the configurations of every batch since the last reset (1.3 MB at 6x6,
+    # 8192 walkers, 20 batches)
+    store = torch.empty(max(1, hparams.num_batches_per_epoch), local_batch, _native.n_words(n_sites),
+                        dtype=torch.int64, device=model.device)
+    state = {'reduced': False, 'stored': 0}
+    diag_shift = float(hparams.sr_diag_shift)
+    tolerance, max_iterations = float(hparams.sr_cg_tolerance), int(hparams.sr_cg_max_iterations)
+    n_sweep_steps = hparams.num_monte_carlo_sweeps * n_sites
+    graphed = {}
+
+    def record():
+      """Stores the configurations the next accumulation sees, on the stream
+      that accumulation runs on."""
+      k = state['stored']
+      if k == store.shape[0]:
+        raise RuntimeError('StochasticReconfiguration keeps %d batches (num_batches_per_epoch) per update: '
+                           'apply or reset the gradients first' % k)
+      store[k].copy_(configs.packed)
+      state['stored'] = k + 1
+
+    def accumulate():
+      record()
+      sums.accumulate(ham, configs.packed)
+      state['reduced'] = False
+
+    def batch_step():
+      """accumulate_gradients followed by one sweep group, as one replayed
+      CUDA graph around cgsvmc_batch_step."""
+      if 'g' not in graphed:
+        graphed['g'] = engine.GraphedBatchStep(configs.state, ansatz, ham, sums, n_sweep_steps)
+      record()
+      graphed['g'].replay()
+      state['reduced'] = False
+
+    def reduce_once():
+      if total is not sums and not state['reduced']:
+        distributed.allreduce_sums(sums.sums, sums.stats, total.sums, total.stats)
+      state['reduced'] = True
+
+    def solve():
+      if state['stored'] == 0:
+        raise RuntimeError('StochasticReconfiguration: no batch accumulated since the last reset')
+      reduce_once()
+      m = total.stats[2]
+      s0, s1 = total.sums[0].double(), total.sums[1].double()
+      o_mean = s0 / m
+      forces = (s1 - total.stats[0] / m * s0) / m
+      packed = store[:state['stored']].reshape(-1, store.shape[2])
+      delta, self.cg_iterations, self.cg_residual = conjugate_gradient(
+          lambda v: sr_matvec(ansatz, packed, o_mean, v, m, diag_shift), forces, tolerance, max_iterations)
+      self.direction = delta
+      return delta
+
+    def apply_gradients():
+      model.apply_gradients(solve().float())
+
+    def metrics():
+      reduce_once()
+      return float((total.stats[0] / total.stats[2]).item())
+
+    def reset():
+      sums.reset()
+      state['reduced'] = False
+      state['stored'] = 0
+
+    self.sums, self.sample_store, self.cg_iterations, self.cg_residual = sums, store, None, None
+    self._batch_step, self._state = Op(batch_step, 'batch_step'), state
+    return TrainOpsTraditional(
+        accumulate_gradients=Op(accumulate, 'accumulate_gradients'),
+        apply_gradients=Op(apply_gradients, 'apply_gradients'),
+        reset_gradients=Op(reset, 'reset_gradients'),
+        mc_step=mc_step, acc_rate=acc_rate,
+        metrics=Op(metrics, 'mean_energy'),
+        epoch_increment=_epoch_increment(),
+        update_wf_norm=_update_norm_op(wavefunction, configs))
+
+  def stored_configs(self):
+    """The configurations accumulated since the last reset, int64 [M_local, W]."""
+    return self.sample_store[:self._state['stored']].reshape(-1, self.sample_store.shape[2])
+
+  def run_optimization_epoch(self, train_ops, session, hparams, epoch_number=0):
+    """EnergyGradientOptimizer's epoch with the SR update; returns the mean
+    energy of the epoch's samples."""
+    session.run(train_ops.mc_step,
+                n_steps=hparams.num_equilibration_sweeps * hparams.num_sites)
+    if train_ops.update_wf_norm is not None:
+      session.run(train_ops.update_wf_norm)
+    session.run(train_ops.reset_gradients)
+    for _ in range(hparams.num_batches_per_epoch):
+      session.run(self._batch_step)
+    session.run(train_ops.apply_gradients)
+    energy = session.run(train_ops.metrics)
+    session.run(train_ops.reset_gradients)
     session.run(train_ops.epoch_increment)
     return energy
 
@@ -776,6 +971,23 @@ GROUND_STATE_OPTIMIZERS = {     # training.py:913-917
                         'raises AttributeError at graph build in the reference '
                         '(hparams.time_evolution_befta, training.py:812)'),
 }
+
+# Ground-state optimizers the reference does not have.  They are kept apart so
+# that GROUND_STATE_OPTIMIZERS names exactly what the reference registers;
+# ground_state_optimizer() and run_training.py --optimizer take both.
+EXTRA_GROUND_STATE_OPTIMIZERS = {
+    'StochasticReconfiguration': StochasticReconfigurationOptimizer,
+}
+
+
+def ground_state_optimizer(name):
+  """The ground-state optimizer class registered under `name`."""
+  if name in GROUND_STATE_OPTIMIZERS:
+    return GROUND_STATE_OPTIMIZERS[name]
+  if name in EXTRA_GROUND_STATE_OPTIMIZERS:
+    return EXTRA_GROUND_STATE_OPTIMIZERS[name]
+  raise KeyError('unknown ground-state optimizer %r: one of %s' % (
+      name, sorted(GROUND_STATE_OPTIMIZERS) + sorted(EXTRA_GROUND_STATE_OPTIMIZERS)))
 
 SUPERVISED_OPTIMIZERS = {       # training.py:920-925
     'SWO': SupervisedWavefunctionOptimizer,

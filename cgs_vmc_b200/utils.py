@@ -111,6 +111,9 @@ def create_hparams(**kwargs):
       learning_rates=[1e-3, 1e-4, 2e-5, 1e-5], learning_rate_stops=[300, 600, 1000],
       optimizer='adam', beta2=0.99,
       num_evaluation_samples=100,
+      # StochasticReconfiguration (not in the reference): shift on the identity,
+      # conjugate-gradient iteration cap and relative residual target
+      sr_diag_shift=0.01, sr_cg_max_iterations=100, sr_cg_tolerance=1e-4,
   )
   hparams.override_from_dict(kwargs)
   return hparams

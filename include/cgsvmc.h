@@ -248,6 +248,20 @@ int cgsvmc_weighted_grad_sum(const cgsvmc_ansatz* ansatz,
                              int64_t n_walkers, int32_t n_weights, float* out,
                              void* stream);
 
+/* The forward counterpart of cgsvmc_weighted_grad_sum (a Jacobian-vector
+ * product of z):
+ *   jvp_out[b] = sum_p (d z_b / d params_p) * tangent[p]   (flat layout, float32 [P])
+ * With it the stochastic-reconfiguration matrix S = <O O^T> - <O><O>^T is
+ * applied to a vector without forming S or the per-walker gradients: one call
+ * here, one cgsvmc_weighted_grad_sum with the centred result as weights.
+ * Built for the pure RBM (rbm with no hidden layers, H <= 256, 1, 2 or 4 spin
+ * words); any other ansatz returns CGSVMC_ERR_UNSUPPORTED, also with
+ * n_walkers == 0, so a call without walkers probes for support.  FP32 with a
+ * fixed summation order (deterministic). */
+int cgsvmc_log_amp_jvp(const cgsvmc_ansatz* ansatz, const uint64_t* packed,
+                       int64_t n_walkers, const float* tangent, float* jvp_out,
+                       void* stream);
+
 /* Replaces one session.run(accumulate_gradients) of
  * EnergyGradientOptimizer (training.py:539-558, 615) in a single pass over the
  * walkers: psi and local energy of every walker (operators.py:249-259), then

@@ -21,7 +21,8 @@ flags.DEFINE_boolean('resume_training', False, 'Restore variables from the lates
 flags.DEFINE_string('wavefunction_type', '', 'Key of wavefunctions.WAVEFUNCTION_TYPES.')
 flags.DEFINE_string('optimizer', 'EnergyGradient',
                     'Key of training.GROUND_STATE_OPTIMIZERS (the reference default ITSWO '
-                    'crashes at graph build, training.py:812).')
+                    'crashes at graph build, training.py:812) or of '
+                    'training.EXTRA_GROUND_STATE_OPTIMIZERS (StochasticReconfiguration).')
 flags.DEFINE_boolean('generate_vectors', False, 'Not available on this path.')
 flags.DEFINE_string('basis_file_path', '', 'Path to the basis file (unused).')
 flags.DEFINE_string('hparams', '', 'Comma-separated name=value overrides.')
@@ -51,7 +52,7 @@ def main(argv):
   bonds, j_x, j_z = drivers.load_bonds(FLAGS.checkpoint_dir, hparams.num_sites, FLAGS.heisenberg_jx)
   wavefunction = wavefunctions.build_wavefunction(hparams)
   hamiltonian = operators.HeisenbergHamiltonian(bonds, j_x, j_z)
-  wavefunction_optimizer = training.GROUND_STATE_OPTIMIZERS[FLAGS.optimizer]()
+  wavefunction_optimizer = training.ground_state_optimizer(FLAGS.optimizer)()
   shared_resources = {}
   train_ops = wavefunction_optimizer.build_opt_ops(
       wavefunction=wavefunction, hamiltonian=hamiltonian, hparams=hparams,
