@@ -128,6 +128,31 @@ __device__ __forceinline__ float group_sum(float v) {
   return v;
 }
 
+// TMA bulk copies global -> shared of `bytes` (a multiple of 16) completing on
+// the mbarrier at shared address bar_a (issued by one thread; the caller has
+// armed the barrier with the expected byte count)
+__device__ __forceinline__ void bulk_copy(void* dst, const void* src, uint32_t bytes, uint32_t bar_a) {
+  char* d = reinterpret_cast<char*>(dst);
+  const char* g = reinterpret_cast<const char*>(src);
+  for (uint32_t done = 0; done < bytes;) {
+    const uint32_t chunk = min(bytes - done, 32768u);
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                     smem_u32(d + done)),
+                 "l"(g + done), "r"(chunk), "r"(bar_a)
+                 : "memory");
+    done += chunk;
+  }
+}
+
+__device__ __forceinline__ void mbar_wait(uint32_t bar_a, uint32_t parity) {
+  uint32_t ok = 0;
+  while (!ok)
+    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                 : "=r"(ok)
+                 : "r"(bar_a), "r"(parity)
+                 : "memory");
+}
+
 // TMA bulk copy global -> shared of the parameter image; every thread returns
 // after the bytes have landed.  `bar` is an 8-byte shared mbarrier.
 // (a second region -- the bond-pair table -- may ride on the same barrier)
@@ -145,30 +170,11 @@ __device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t b
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a),
                  "r"(bytes + bytes2 + bytes3)
                  : "memory");
-    for (int region = 0; region < 3; ++region) {
-      char* d = reinterpret_cast<char*>(region == 0 ? dst : region == 1 ? dst2 : dst3);
-      const char* g = reinterpret_cast<const char*>(region == 0 ? src : region == 1 ? src2 : src3);
-      const uint32_t total = region == 0 ? bytes : region == 1 ? bytes2 : bytes3;
-      uint32_t done = 0;
-      while (done < total) {
-        const uint32_t chunk = min(total - done, 32768u);
-        asm volatile(
-            "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                smem_u32(d + done)),
-            "l"(g + done), "r"(chunk), "r"(bar_a)
-            : "memory");
-        done += chunk;
-      }
-    }
+    bulk_copy(dst, src, bytes, bar_a);
+    bulk_copy(dst2, src2, bytes2, bar_a);
+    bulk_copy(dst3, src3, bytes3, bar_a);
   }
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-        : "=r"(ok)
-        : "r"(bar_a), "r"(0u)
-        : "memory");
-  }
+  mbar_wait(bar_a, 0u);
 }
 
 // select-in-byte table: lut[v * 8 + r] = index of the r-th set bit of v
@@ -1004,8 +1010,9 @@ __device__ __forceinline__ void grid_reduce(const WalkerArgs& A, float* red) {
 // kernel is shared-memory bandwidth); to make room the shared-memory image
 // starts at the F table and the 2W rows of the state build are parked in the
 // buffer that later stages tanh(theta) for the gradient tiles (a CTA barrier
-// separates the two uses; later batches of the same CTA read 2W from global
-// memory).
+// separates the two uses).  With the gradient on the tensor cores the rows are
+// copied back during every pass's sweep, once the MMAs have read the staged
+// operands; otherwise later batches of the same CTA read 2W from global memory.
 template <int NW, int LPW, int KJV, bool WS, bool MC, bool PT = false>
 __global__ void __launch_bounds__((Geometry<LPW, KJV, true>::THREADS), 1)
 walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
@@ -1018,12 +1025,12 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
   const int img_skip = PT ? im.off_f : 0;          // floats of the image left in global memory
   float* img_s = smem - img_skip;                  // so that img_s + off_x addresses table x
   char* cur = reinterpret_cast<char*>(smem + (WS ? im.total - img_skip : 0));
-  uint64_t* bar = reinterpret_cast<uint64_t*>(cur); cur += 32;   // table mbarrier, tile counter, MMA mbarrier, TMEM address
+  uint64_t* bar = reinterpret_cast<uint64_t*>(cur); cur += 32;   // table mbarrier, tile counter, TMEM address, MMA mbarrier, 2W mbarrier
   int4* bond_s = reinterpret_cast<int4*>(cur); cur += (size_t)(A.do_eloc ? A.n_bonds : 0) * 16;
   const int list_ld = (A.n_bonds + 7) / 8 * 8;
   uint32_t* list_s = reinterpret_cast<uint32_t*>(cur); cur += (size_t)(A.do_eloc ? SLOTS * list_ld : 0) * 4;
   const int NP4 = (im.N + 1 + 3) / 4 * 4;
-  // (PT: at least N rows, the first batch's 2W table lives here during the state build)
+  // (PT: at least N rows, the 2W table lives here during the state build)
   float* T_s = reinterpret_cast<float*>(cur);
   cur += (size_t)max(A.do_grad ? SLOTS * HP : 0, PT ? im.N * HP : 0) * 4;
   float* ws_s = reinterpret_cast<float*>(cur); cur += (size_t)(A.do_grad ? SLOTS * 2 * NP4 : 0) * 4;
@@ -1036,6 +1043,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
   const float* pair_s = PT ? reinterpret_cast<const float*>(cur) : (!WS ? A.pair_table : nullptr);
   int* tile_next_s = reinterpret_cast<int*>(bar) + 2;                // behind the 8-byte mbarrier
   uint64_t* mma_bar = bar + 2;
+  uint64_t* w2_bar = bar + 3;                                        // 2W rows parked in T_s again (tcg)
   uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(bar) + 3;
   // ---- gradient sums on the tensor cores (PT kernels, A.tc_grad) ----
   // S_k[i][j] = sum_b (w_kb sigma_bi) tanh(theta_bj) is a GEMM over the walkers
@@ -1096,6 +1104,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
   if (tcg) {
     if (threadIdx.x == 0) {
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mma_bar)) : "memory");
+      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(w2_bar)) : "memory");
       asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
@@ -1115,8 +1124,10 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
     tmem = *tmem_holder;
   }
   RBM2_MARK(1, 1);
+  // t.w2: the 2W rows outside the state build at the top of a pass (the
+  // sampler's rare state rebuild); with the gradient T_s holds staged operands then
   Tables t = tables_at(WS ? img_s : img_g, im);
-  if (PT) t.w2 = T_s;
+  if (PT) t.w2 = A.do_grad ? img_g + im.off_w2 : T_s;
   SitePicker<NW, LPW> picker;
   if (MC) picker.setup(im.N, sub);
   unsigned int n_acc = 0;
@@ -1155,6 +1166,11 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
     const int64_t ob = (int64_t)iter * A.out_stride + b;      // row of this pass in e_loc / log_amp / diag / off
     RBM2_MARK(1, 10);
     float p[KJ], m[KJ];
+    // PT: the state build reads the 2W rows parked in T_s -- without the
+    // gradient T_s holds nothing else, the first pass finds them there from the
+    // table copy, and with the gradient on the tensor cores the previous pass
+    // has copied them back (w2_bar)
+    const bool w2_parked = PT && (!A.do_grad || batch_no == 0 || tcg);
     if (warp_on) {
       if (batch_no == 0) {
 #pragma unroll
@@ -1167,44 +1183,41 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
         for (int w = 0; w < NW; ++w) s[w] = w < im.words ? __ldcg(A.packed_rw + bb * im.words + w) : 0ull;
       }
       const bool want_z = A.log_amp != nullptr;
-      float z = init_state<NW, LPW, KJV, WS>(t, im, s, sub, p, m, want_z);
+      if (tcg && batch_no > 0) mbar_wait(smem_u32(w2_bar), (uint32_t)(batch_no - 1) & 1u);
+      Tables tb = t;
+      if (w2_parked) tb.w2 = T_s;
+      float z = init_state<NW, LPW, KJV, WS>(tb, im, s, sub, p, m, want_z);
       if (want_z) {
         z = group_sum<LPW>(z) + ld1<WS>(t.a0);
         if (valid && sub == 0) A.log_amp[ob] = z;
       }
       RBM2_MARK(1, 2);
     }
-    // PT: every warp is done with the parked 2W rows before T_s is written for
-    // the gradient; from here on (the sampler's rare state rebuild, later
-    // batches) the 2W rows come from global memory
-    if (PT && A.do_grad && batch_no == 0) {
-      __syncthreads();
-      t.w2 = img_g + im.off_w2;
-      if (tcg) {      // B planes: rows of empty slots stay zero (finite) for the whole launch
-        for (int e = threadIdx.x; e < SLOTS * HP / 4; e += THREADS)
-          reinterpret_cast<uint4*>(T_s)[e] = make_uint4(0u, 0u, 0u, 0u);
-        __syncthreads();
-      }
-    }
+    // every warp is done with the parked 2W rows before T_s is written for the gradient
+    if (A.do_grad && w2_parked) __syncthreads();
     // the MMAs of the previous pass have read the operand planes; a full
     // segment of kTcgSegment passes is drained before the next one starts
     // (bounds the truncating accumulation in TMEM)
     const bool seg_start = tcg && (batch_no % kTcgSegment) == 0;
     if (tcg && batch_no > 0) {
-      const uint32_t bar_a = smem_u32(mma_bar), parity = (uint32_t)(batch_no - 1) & 1u;
-      uint32_t ok = 0;
-      while (!ok)
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(bar_a), "r"(parity) : "memory");
+      mbar_wait(smem_u32(mma_bar), (uint32_t)(batch_no - 1) & 1u);
       if (seg_start) {
         tcg_drain<THREADS, NCOL>(tmem, T_s, drain_groups, part, A.P, im.N, im.H, NC, n_drained > 0);
         ++n_drained;
         // the staging went through the operand planes: rows of empty slots must read as zero again
-        for (int e = threadIdx.x; e < SLOTS * HP / 4; e += THREADS)
-          reinterpret_cast<uint4*>(T_s)[e] = make_uint4(0u, 0u, 0u, 0u);
         for (int e = threadIdx.x; e < SLOTS * 2 * NP4 / 4; e += THREADS)
           reinterpret_cast<uint4*>(ws_s)[e] = make_uint4(0u, 0u, 0u, 0u);
         __syncthreads();
+      }
+    }
+    if (tcg) {
+      // B planes: rows of slots without a walker must read as zero (finite); the
+      // 2W rows or the drain staging were there
+      const int n_empty = SLOTS - n_valid;
+      for (int e = threadIdx.x; e < n_empty * 2 * NB; e += THREADS) {
+        const int ch = e / n_empty, sl = n_valid + e % n_empty;
+        *reinterpret_cast<uint4*>(reinterpret_cast<char*>(T_s) + ((size_t)ch * SLOTS + sl) * 16) =
+            make_uint4(0u, 0u, 0u, 0u);
       }
     }
     float e_val = 0.f;
@@ -1408,6 +1421,19 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
       __syncwarp();        // a later iteration of this lane group may read the words back
       RBM2_MARK(1, 5);
     }
+    // once the MMAs of this pass have read the operand planes, the MMA warp parks
+    // the 2W rows in T_s again for the next pass's state build (during the sweep:
+    // at C2 the last warp owns no walker)
+    if (tcg && warp == THREADS / 32 - 1 && (batch + gridDim.x < A.n_batches || iter + 1 < n_iters)) {
+      mbar_wait(smem_u32(mma_bar), (uint32_t)batch_no & 1u);
+      if (lane == 0) {
+        const uint32_t bytes = (uint32_t)(im.N * HP) * 4u;
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(w2_bar)), "r"(bytes)
+                     : "memory");
+        bulk_copy(T_s, img_g + im.off_w2, bytes, smem_u32(w2_bar));
+      }
+      __syncwarp();
+    }
     if (A.do_grad) {
       RBM2_MARK(1, 6);
       // side sums first (the warps at the END of the CTA get here early)
@@ -1525,11 +1551,7 @@ walker_kernel(Image im, const float* __restrict__ img_g, WalkerArgs A) {
   }
   if (tcg && batch_no > 0) {
     // the passes since the last drain are still in TMEM
-    const uint32_t bar_a = smem_u32(mma_bar), parity = (uint32_t)(batch_no - 1) & 1u;
-    uint32_t ok = 0;
-    while (!ok)
-      asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                   : "=r"(ok) : "r"(bar_a), "r"(parity) : "memory");
+    mbar_wait(smem_u32(mma_bar), (uint32_t)(batch_no - 1) & 1u);
     tcg_drain<THREADS, NCOL>(tmem, T_s, drain_groups, part, A.P, im.N, im.H, NC, n_drained > 0);
   }
   if (A.do_grad) {
