@@ -32,8 +32,13 @@ EXPORTS = [
     'cgsvmc_propose_exchange', 'cgsvmc_accept_exchange', 'cgsvmc_local_energy_from_amps',
     'cgsvmc_swo_weights', 'cgsvmc_adam_step', 'cgsvmc_batch_step_fed', 'cgsvmc_batch_steps',
     'cgsvmc_epoch_end', 'cgsvmc_pack_configs_host', 'cgsvmc_upload_configs',
-    'cgsvmc_conv_periodic', 'cgsvmc_log_amp_jvp',
+    'cgsvmc_conv_periodic', 'cgsvmc_log_amp_jvp', 'cgsvmc_rbm2_plan',
 ]
+# cgsvmc_rbm2_plan: entry points (modes) and the fields it reports, in order
+RBM2_PLAN_MODES = {'mc_steps': 0, 'local_energy': 1, 'weighted_grad_sum': 2, 'accumulate': 3,
+                   'batch_step': 4, 'batch_steps': 4}
+RBM2_PLAN_FIELDS = ('supported', 'nw', 'lpw', 'kjv', 'slots', 'wpc', 'n_batches', 'grid', 'tables_in_smem',
+                    'pair_table', 'tc_grad', 'fused_reduce', 'keeps_walkers')
 
 
 class AnsatzDesc(ctypes.Structure):
@@ -82,6 +87,7 @@ def load():
   lib.cgsvmc_local_energy.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, vp]
   lib.cgsvmc_weighted_grad_sum.argtypes = [vp, vp, vp, i64, i32, vp, vp]
   lib.cgsvmc_log_amp_jvp.argtypes = [vp, vp, i64, vp, vp, vp]
+  lib.cgsvmc_rbm2_plan.argtypes = [vp, vp, i64, i32, vp, i32]
   lib.cgsvmc_energy_stats.argtypes = [vp, i64, vp, vp]
   lib.cgsvmc_accumulate.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, vp]
   lib.cgsvmc_batch_step.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, i32, u64, u64, u64, vp, vp, vp]
@@ -293,6 +299,22 @@ class Ansatz:
       _want(out, torch.float32, (b,), 'out')
     check(load().cgsvmc_log_amp_jvp(self._handle, _ptr(packed), b, _ptr(tangent), _ptr(out), _stream()))
     return out
+
+  def rbm2_plan(self, ham, n_walkers, mode):
+    """The pure-RBM kernel variant that entry point `mode` (a key of
+    RBM2_PLAN_MODES) would run for n_walkers walkers, as a dict of
+    RBM2_PLAN_FIELDS (cgsvmc_rbm2_plan; pair_table: 0 none, 1 shared, 2 global
+    memory), or None when the call takes another path.  Allocates and launches
+    nothing."""
+    if mode not in RBM2_PLAN_MODES:
+      raise ValueError('unknown rbm2 plan mode %r' % (mode,))
+    out = (ctypes.c_int32 * len(RBM2_PLAN_FIELDS))()
+    rc = load().cgsvmc_rbm2_plan(self._handle, None if ham is None else ham._handle, int(n_walkers),
+                                 RBM2_PLAN_MODES[mode], out, len(RBM2_PLAN_FIELDS))
+    if rc == ERR_UNSUPPORTED:
+      return None
+    check(rc)
+    return dict(zip(RBM2_PLAN_FIELDS, (int(v) for v in out)))
 
   def accumulate(self, ham, packed, sums, stats, e_loc_out=None, log_amp_out=None):
     """One session.run(accumulate_gradients) (training.py:539-558): sums [2, P]

@@ -541,6 +541,22 @@ int cgsvmc_batch_steps(const cgsvmc_ansatz* a, const cgsvmc_ham* h, uint64_t* pa
   return CGSVMC_OK;
 }
 
+int cgsvmc_rbm2_plan(const cgsvmc_ansatz* a, const cgsvmc_ham* h, int64_t B, int32_t mode, int32_t* out,
+                     int32_t n_out) {
+  if (a == nullptr) return invalid("ansatz handle is NULL");
+  if (B < 1) return invalid("rbm2_plan: n_walkers < 1");
+  if (n_out < 0 || (n_out > 0 && out == nullptr)) return invalid("rbm2_plan: bad output buffer");
+  if (mode < CGSVMC_RBM2_PLAN_MC_STEPS || mode > CGSVMC_RBM2_PLAN_BATCH_STEPS) return invalid("rbm2_plan: unknown mode");
+  const bool needs_ham = mode == CGSVMC_RBM2_PLAN_LOCAL_ENERGY || mode == CGSVMC_RBM2_PLAN_ACCUMULATE ||
+                         mode == CGSVMC_RBM2_PLAN_BATCH_STEPS;
+  if (needs_ham && h == nullptr) return invalid("rbm2_plan: NULL hamiltonian");
+  if (needs_ham && h->n_sites != a->desc.n_sites) return invalid("rbm2_plan: hamiltonian and ansatz n_sites differ");
+  int32_t fields[kRbm2PlanFields];
+  const int rc = rbm2_plan(a, needs_ham ? h : nullptr, B, mode, fields);
+  for (int i = 0; i < n_out && i < kRbm2PlanFields; ++i) out[i] = fields[i];
+  return rc;
+}
+
 int cgsvmc_batch_step_fed(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const float* configs_f32,
                           uint64_t* packed_out, int64_t B, float* e_loc_out, float* log_amp_out,
                           float* sums, double* stats, int32_t n_steps, uint64_t seed, uint64_t walker_id0,

@@ -140,6 +140,11 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
                 float* e_loc, float* log_amp, float* diag, float* off, bool do_grad,
                 const float* weights, int K, float* out, double* stats, cudaStream_t s,
                 const Rbm2Sweep* sweep = nullptr);
+// The launch plan of the entry point `mode` (CGSVMC_RBM2_PLAN_*) for B walkers,
+// in the field order of cgsvmc_rbm2_plan; CGSVMC_ERR_UNSUPPORTED when rbm2 does
+// not take the call.  No allocation, no launch.
+constexpr int kRbm2PlanFields = 13;
+int rbm2_plan(const cgsvmc_ansatz* a, const cgsvmc_ham* h, int64_t B, int mode, int32_t (&out)[kRbm2PlanFields]);
 
 // ---- conv_1d / conv_2d forward on the tensor cores (conv_tc.cu): tcgen05 + TMEM ----
 bool conv_tc_supported(const cgsvmc_ansatz* a, const cgsvmc_ham* h);

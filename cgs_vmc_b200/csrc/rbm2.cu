@@ -212,12 +212,20 @@ int build_image(cgsvmc_ansatz* a, const Plan& pl, cudaStream_t st) {
   return cuda_fail(cudaGetLastError(), "rbm2 prep launch");
 }
 
+// Whether pair_slot can give (ansatz, Hamiltonian) a slot of `bytes`: the
+// Hamiltonian has one that large, or there is room for another.  Allocates nothing.
+bool pair_slot_possible(const cgsvmc_ansatz* a, const cgsvmc_ham* h, size_t bytes) {
+  for (const auto& pt : a->pair_tables)
+    if (pt.ham_uid == h->uid) return pt.bytes >= bytes;
+  return (int)a->pair_tables.size() < cgsvmc_ansatz::kMaxPairTables;
+}
+
 // The pair-table slot of (ansatz, Hamiltonian); nullptr when the ansatz has
 // already been used with kMaxPairTables other Hamiltonians.
 cgsvmc_ansatz::PairTable* pair_slot(cgsvmc_ansatz* a, const cgsvmc_ham* h, size_t bytes) {
+  if (!pair_slot_possible(a, h, bytes)) return nullptr;
   for (auto& pt : a->pair_tables)
-    if (pt.ham_uid == h->uid) return pt.bytes >= bytes ? &pt : nullptr;
-  if ((int)a->pair_tables.size() >= cgsvmc_ansatz::kMaxPairTables) return nullptr;
+    if (pt.ham_uid == h->uid) return &pt;
   cgsvmc_ansatz::PairTable pt;
   pt.ham_uid = h->uid;
   if (cudaMalloc(&pt.buf, bytes) != cudaSuccess) { cudaGetLastError(); return nullptr; }
@@ -233,6 +241,74 @@ int build_pair_table(cgsvmc_ansatz* a, const cgsvmc_ham* h, const Plan& pl,
   pair_prep_kernel<<<2 * h->n_bonds, 128, 0, st>>>(pl.im, a->tables, h->ij, h->n_bonds, slot->buf);
   slot->valid = true;
   return cuda_fail(cudaGetLastError(), "rbm2 pair prep launch");
+}
+
+// Launch plan of the sampler kernel (rbm2_mc_steps).
+int plan_mc(const cgsvmc_ansatz* a, int64_t B, Plan* pl) {
+  if (!base_plan(a, B, pl, false)) { set_error("rbm2: unsupported ansatz"); return CGSVMC_ERR_UNSUPPORTED; }
+  const size_t img_bytes = (size_t)pl->im.total * 4;
+  pl->ws = img_bytes + 16 <= (size_t)a->max_smem_optin;
+  pl->pt = pl->pt_global = pl->tc_grad = pl->fuse = false;
+  pl->mc_smem = (pl->ws ? img_bytes : 2048) + 16;
+  pl->walker_smem = 0;
+  pl->step0_dev = nullptr;
+  return CGSVMC_OK;
+}
+
+// Launch plan of the walker kernel (rbm2_walker): table placement, bond-pair
+// table, tensor-core gradient and in-kernel reduction.  Depends only on the
+// shape, the device, the pair-table slots the ansatz already holds and the
+// environment switches; allocates and launches nothing, so that
+// cgsvmc_rbm2_plan reports what a call would run.  `no_pair_table` plans the
+// two-row path (the pair-table allocation failed).
+int plan_walker(const cgsvmc_ansatz* a, const cgsvmc_ham* h, int64_t B, bool do_grad, bool weighted, bool mc,
+                bool no_pair_table, Plan* pl) {
+  if (!base_plan(a, B, pl, true)) { set_error("rbm2: unsupported ansatz"); return CGSVMC_ERR_UNSUPPORTED; }
+  const bool do_eloc = h != nullptr;
+  const int slots = pl->slots;
+  const int nb = do_eloc ? h->n_bonds : 0;
+  pl->ws = walker_smem_bytes(pl->im, slots, true, do_eloc, nb, do_grad, mc) <= (size_t)a->max_smem_optin;
+  const bool pair_ok = !no_pair_table && do_eloc && nb >= 1 && nb < 16384 &&
+                       pair_slot_possible(a, h, (size_t)2 * nb * pl->im.HP * 4);
+  // bond-pair table: 8 lanes per walker, at least one bond, pair index below 2^15,
+  // and everything (image from F on + pair table + staging) in shared memory
+  pl->pt = pair_ok && pl->ws && pl->lpw == 8 &&
+           walker_smem_bytes(pl->im, slots, true, do_eloc, nb, do_grad, mc, true) <= (size_t)a->max_smem_optin;
+  // tables in global memory: the pair table too (read through L1 / L2)
+  pl->pt_global = pair_ok && !pl->ws;
+  pl->walker_smem = walker_smem_bytes(pl->im, slots, pl->ws, do_eloc, nb, do_grad, mc, pl->pt);
+  pl->mc_smem = 0;
+  pl->step0_dev = nullptr;
+  if (pl->walker_smem > (size_t)a->max_smem_optin) {
+    set_error("rbm2: problem does not fit in shared memory");
+    return CGSVMC_ERR_UNSUPPORTED;
+  }
+  // gradient sums on the tensor cores: pair-table kernels with weights (1, E_loc),
+  // sigma + three weight pieces within M = 128 rows (N <= 39), a spare column for
+  // the constant 1 (H < HP), operand planes no larger than the float staging
+  // buffers they replace.  CGSVMC_RBM2_TC_GRAD=0 keeps the FP32 register tiles.
+  // (read at every call so that tests can compare the two paths)
+  {
+    const char* e = getenv("CGSVMC_RBM2_TC_GRAD");
+    const bool off = e != nullptr && atoi(e) == 0;
+    const int np4 = round_up(pl->im.N + 1, 4), np8 = round_up(pl->im.N + 1, 8);
+    pl->tc_grad = !off && pl->pt && do_grad && !weighted && np8 == np4 && 3 * np8 <= 128 &&
+                  pl->im.H < pl->im.HP && 3 * pl->im.HP <= 512 && (slots == 64 || slots == 128);
+  }
+  // The cross-CTA reduction runs inside the walker kernel when the device can
+  // launch it cooperatively (all CTAs co-resident: grid <= number of SMs, one
+  // CTA per SM) and the staging buffer is large enough for its scratch.
+  // CGSVMC_RBM2_FUSED_REDUCE=0 keeps the separate reduction kernel.
+  const char* fuse_env = getenv("CGSVMC_RBM2_FUSED_REDUCE");
+  const bool fuse_off = fuse_env != nullptr && atoi(fuse_env) == 0;
+  pl->fuse = false;
+  if (do_grad && !fuse_off && pl->grid <= a->num_sms) {
+    int coop = 0;
+    cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, a->device);
+    const int threads = variant_slots(pl->lpw, pl->kjv, true) / (32 / pl->lpw) * 32;
+    pl->fuse = coop != 0 && (size_t)slots * pl->im.HP >= (size_t)(threads / 32) * 96;
+  }
+  return CGSVMC_OK;
 }
 
 }  // namespace
@@ -254,10 +330,7 @@ int rbm2_mc_steps(cgsvmc_ansatz* a, uint64_t* packed, int64_t B, int n_steps, ui
                   uint64_t walker0, uint64_t step0, unsigned long long* accept_count,
                   float* log_amp_out, cudaStream_t st) {
   Plan pl;
-  if (!base_plan(a, B, &pl, false)) { set_error("rbm2: unsupported ansatz"); return CGSVMC_ERR_UNSUPPORTED; }
-  const size_t img_bytes = (size_t)pl.im.total * 4;
-  pl.ws = img_bytes + 16 <= (size_t)a->max_smem_optin;
-  pl.mc_smem = (pl.ws ? img_bytes : 2048) + 16;
+  if (int rc = plan_mc(a, B, &pl)) return rc;
   pl.step0_dev = a->step_counter_dev;
   if (int rc = build_image(a, pl, st)) return rc;
   switch (pl.nw) {
@@ -271,27 +344,15 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
                 float* e_loc, float* log_amp, float* diag, float* off, bool do_grad,
                 const float* weights, int K, float* out, double* stats, cudaStream_t st,
                 const Rbm2Sweep* sweep) {
-  Plan pl;
-  if (!base_plan(a, B, &pl, true)) { set_error("rbm2: unsupported ansatz"); return CGSVMC_ERR_UNSUPPORTED; }
   const bool do_eloc = h != nullptr;
   const bool mc = sweep != nullptr;
-  const int slots = pl.slots;
+  Plan pl;
+  if (int rc = plan_walker(a, h, B, do_grad, weights != nullptr, mc, false, &pl)) return rc;
   const int nb = do_eloc ? h->n_bonds : 0;
-  pl.ws = walker_smem_bytes(pl.im, slots, true, do_eloc, nb, do_grad, mc) <= (size_t)a->max_smem_optin;
-  // bond-pair table: 8 lanes per walker, at least one bond, pair index below 2^15,
-  // and everything (image from F on + pair table + staging) in shared memory
-  pl.pt = do_eloc && pl.ws && pl.lpw == 8 && nb >= 1 && nb < 16384 &&
-          walker_smem_bytes(pl.im, slots, true, do_eloc, nb, do_grad, mc, true) <= (size_t)a->max_smem_optin;
-  // tables in global memory: the pair table too (read through L1 / L2)
-  const bool pt_global = do_eloc && !pl.ws && nb >= 1 && nb < 16384;
   cgsvmc_ansatz::PairTable* slot =
-      (pl.pt || pt_global) ? pair_slot(a, h, (size_t)2 * nb * pl.im.HP * 4) : nullptr;
-  if (slot == nullptr) pl.pt = false;
-  pl.walker_smem = walker_smem_bytes(pl.im, slots, pl.ws, do_eloc, nb, do_grad, mc, pl.pt);
-  if (pl.walker_smem > (size_t)a->max_smem_optin) {
-    set_error("rbm2: problem does not fit in shared memory");
-    return CGSVMC_ERR_UNSUPPORTED;
-  }
+      (pl.pt || pl.pt_global) ? pair_slot(a, h, (size_t)2 * nb * pl.im.HP * 4) : nullptr;
+  if ((pl.pt || pl.pt_global) && slot == nullptr)      // the allocation failed: the two-row path
+    if (int rc = plan_walker(a, h, B, do_grad, weights != nullptr, mc, true, &pl)) return rc;
   if (int rc = build_image(a, pl, st)) return rc;
   if (slot != nullptr)
     if (int rc = build_pair_table(a, h, pl, slot, st)) return rc;
@@ -310,35 +371,12 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
     A.n_steps = sweep->n_steps; A.seed = sweep->seed; A.walker0 = sweep->walker0;
     A.step0 = sweep->step0; A.step0_dev = a->step_counter_dev; A.accept_count = sweep->accept_count;
   }
-  // gradient sums on the tensor cores: pair-table kernels with weights (1, E_loc),
-  // sigma + three weight pieces within M = 128 rows (N <= 39), a spare column for
-  // the constant 1 (H < HP), operand planes no larger than the float staging
-  // buffers they replace.  CGSVMC_RBM2_TC_GRAD=0 keeps the FP32 register tiles.
-  {
-    const char* e = getenv("CGSVMC_RBM2_TC_GRAD");
-    const bool off = e != nullptr && atoi(e) == 0;
-    const int np4 = round_up(pl.im.N + 1, 4), np8 = round_up(pl.im.N + 1, 8);
-    A.tc_grad = (!off && pl.pt && do_grad && weights == nullptr && np8 == np4 && 3 * np8 <= 128 &&
-                 pl.im.H < pl.im.HP && 3 * pl.im.HP <= 512 && (slots == 64 || slots == 128)) ? 1 : 0;
-  }
+  A.tc_grad = pl.tc_grad ? 1 : 0;
   if (mc) A.configs_f32 = sweep->configs_f32;
   const int n_iters = mc && sweep->n_iters > 1 ? sweep->n_iters : 1;
   A.n_iters = n_iters;
   A.out_stride = n_iters > 1 ? B : 0;
-  // The cross-CTA reduction runs inside the walker kernel when the device can
-  // launch it cooperatively (all CTAs co-resident: grid <= number of SMs, one
-  // CTA per SM) and the staging buffer is large enough for its scratch.
-  // CGSVMC_RBM2_FUSED_REDUCE=0 keeps the separate reduction kernel.
-  // (read at every call so that tests can compare the two paths)
-  const char* fuse_env = getenv("CGSVMC_RBM2_FUSED_REDUCE");
-  const bool fuse_off = fuse_env != nullptr && atoi(fuse_env) == 0;
-  bool fuse = false;
-  if (do_grad && !fuse_off && pl.grid <= a->num_sms) {
-    int coop = 0;
-    cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, a->device);
-    const int threads = variant_slots(pl.lpw, pl.kjv, true) / (32 / pl.lpw) * 32;
-    fuse = coop != 0 && (size_t)slots * pl.im.HP >= (size_t)(threads / 32) * 96;
-  }
+  const bool fuse = pl.fuse;
   if (fuse && a->grid_sync == nullptr) {
     if (int rc = cuda_fail(cudaMalloc(&a->grid_sync, 128), "grid_sync alloc")) return rc;
     if (int rc = cuda_fail(cudaMemset(a->grid_sync, 0, 128), "grid_sync clear")) return rc;
@@ -375,6 +413,38 @@ int rbm2_walker(cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, i
                                           snapshot);
     return cuda_fail(cudaGetLastError(), "rbm2 reduce launch");
   }
+  return CGSVMC_OK;
+}
+
+int rbm2_plan(const cgsvmc_ansatz* a, const cgsvmc_ham* h, int64_t B, int mode, int32_t (&out)[kRbm2PlanFields]) {
+  for (int32_t& v : out) v = 0;
+  const bool sampler = mode == CGSVMC_RBM2_PLAN_MC_STEPS;
+  const bool grad_only = mode == CGSVMC_RBM2_PLAN_WEIGHTED_GRAD_SUM;
+  const cgsvmc_ham* hw = sampler || grad_only ? nullptr : h;
+  if (!rbm2_supported(a, hw)) {
+    set_error("rbm2: the call takes another path");
+    return CGSVMC_ERR_UNSUPPORTED;
+  }
+  const bool mc = mode == CGSVMC_RBM2_PLAN_BATCH_STEPS;
+  const bool do_grad = mc || grad_only || mode == CGSVMC_RBM2_PLAN_ACCUMULATE;
+  Plan pl;
+  const int rc = sampler ? plan_mc(a, B, &pl) : plan_walker(a, hw, B, do_grad, grad_only, mc, false, &pl);
+  if (rc) return rc;
+  out[0] = 1;
+  out[1] = pl.nw;
+  out[2] = pl.lpw;
+  out[3] = pl.kjv;
+  out[4] = pl.slots;
+  out[5] = pl.wpc;
+  out[6] = (int32_t)std::min<int64_t>(pl.n_batches, INT32_MAX);
+  out[7] = pl.grid;
+  out[8] = pl.ws ? 1 : 0;
+  out[9] = pl.pt ? 1 : (pl.pt_global ? 2 : 0);
+  out[10] = pl.tc_grad ? 1 : 0;
+  out[11] = pl.fuse ? 1 : 0;
+  // the walker kernel keeps a swept walker in registers for the next iteration
+  // when every CTA has one batch
+  out[12] = mc && pl.n_batches <= (int64_t)pl.grid ? 1 : 0;
   return CGSVMC_OK;
 }
 

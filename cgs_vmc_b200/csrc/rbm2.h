@@ -20,6 +20,9 @@ struct Plan {
   int slots;             // walkers per CTA batch the variant can hold
   bool ws;               // image in shared memory
   bool pt;               // walker kernel: bond-pair table in shared memory (E_loc reads one row per ratio)
+  bool pt_global;        // walker kernel: bond-pair table in global memory (tables too large for shared memory)
+  bool tc_grad;          // walker kernel: gradient sums on the tensor cores
+  bool fuse;             // walker kernel: cross-CTA reduction inside the (cooperative) launch
   int wpc;               // walkers per CTA batch
   int64_t n_batches;
   int grid;

@@ -314,6 +314,29 @@ int cgsvmc_batch_steps(const cgsvmc_ansatz* ansatz, const cgsvmc_ham* ham,
                        uint64_t* step_counter, unsigned long long* accept_count,
                        void* stream);
 
+/* Which variant of the pure-RBM kernels (rbm2) an entry point would run for
+ * n_walkers walkers with the current device, switches and pair-table slots,
+ * without allocating or launching anything.  `mode` names the entry point:
+ * CGSVMC_RBM2_PLAN_MC_STEPS, _LOCAL_ENERGY, _WEIGHTED_GRAD_SUM, _ACCUMULATE or
+ * _BATCH_STEPS (cgsvmc_batch_step and cgsvmc_batch_steps).  `ham` is needed for
+ * LOCAL_ENERGY, ACCUMULATE and BATCH_STEPS and ignored otherwise.  The first
+ * n_out (at most 13) of these fields go to out:
+ *   supported (1), words per walker, lanes per walker, HP / 32, walker slots
+ *   per CTA, walkers per CTA batch, batches, grid, parameter tables in shared
+ *   memory (0/1), bond-pair table (0 none, 1 shared, 2 global memory), gradient
+ *   sums on the tensor cores (0/1), cross-CTA reduction inside the kernel
+ *   (0/1), walkers kept in registers between the iterations of
+ *   cgsvmc_batch_steps (0/1).
+ * Returns CGSVMC_ERR_UNSUPPORTED (out zeroed) when rbm2 does not take the call:
+ * another path serves it. */
+#define CGSVMC_RBM2_PLAN_MC_STEPS 0
+#define CGSVMC_RBM2_PLAN_LOCAL_ENERGY 1
+#define CGSVMC_RBM2_PLAN_WEIGHTED_GRAD_SUM 2
+#define CGSVMC_RBM2_PLAN_ACCUMULATE 3
+#define CGSVMC_RBM2_PLAN_BATCH_STEPS 4
+int cgsvmc_rbm2_plan(const cgsvmc_ansatz* ansatz, const cgsvmc_ham* ham,
+                     int64_t n_walkers, int32_t mode, int32_t* out, int32_t n_out);
+
 /* cgsvmc_batch_step for a caller that holds the walkers in the reference's own
  * layout (the float32 [B, N] variable of graph_builders.py:92-125) and reads
  * the energy statistics back every batch (training.py:619-620): configs_f32
