@@ -33,6 +33,7 @@ EXPORTS = [
     'cgsvmc_swo_weights', 'cgsvmc_adam_step', 'cgsvmc_batch_step_fed', 'cgsvmc_batch_steps',
     'cgsvmc_epoch_end', 'cgsvmc_pack_configs_host', 'cgsvmc_upload_configs',
     'cgsvmc_conv_periodic', 'cgsvmc_log_amp_jvp', 'cgsvmc_rbm2_plan',
+    'cgsvmc_bond_values', 'cgsvmc_bond_values_from_amps',
 ]
 # cgsvmc_rbm2_plan: entry points (modes) and the fields it reports, in order
 RBM2_PLAN_MODES = {'mc_steps': 0, 'local_energy': 1, 'weighted_grad_sum': 2, 'accumulate': 3,
@@ -94,6 +95,8 @@ def load():
   lib.cgsvmc_propose_exchange.argtypes = [vp, i64, i32, u64, u64, u64, vp, vp, vp]
   lib.cgsvmc_accept_exchange.argtypes = [vp, vp, i64, i32, vp, vp, vp, vp, vp, vp, vp]
   lib.cgsvmc_local_energy_from_amps.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp]
+  lib.cgsvmc_bond_values.argtypes = [vp, vp, vp, i64, vp, vp]
+  lib.cgsvmc_bond_values_from_amps.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp]
   f32 = ctypes.c_float
   lib.cgsvmc_batch_steps.argtypes = [vp, vp, vp, i64, i32, vp, vp, vp, vp, i32, u64, u64, u64, vp, vp, vp]
   lib.cgsvmc_batch_step_fed.argtypes = [vp, vp, vp, vp, i64, vp, vp, vp, vp, i32, u64, u64, u64, vp, vp, vp, vp]
@@ -267,6 +270,20 @@ class Ansatz:
     check(load().cgsvmc_local_energy(self._handle, ham._handle, _ptr(packed), b,
                                      _ptr(e), _ptr(z), _ptr(diag), _ptr(off), _stream()))
     return (e, z, diag, off) if want_parts else (e, z)
+
+  def bond_values(self, ham, packed, out=None):
+    """float32 [B, n_bonds]: the per-bond terms of local_energy
+    (cgsvmc_bond_values; pure RBM only, NotImplementedError otherwise -- a call
+    with no walkers probes for support)."""
+    self._sync_params()
+    b = packed.shape[0]
+    _want(packed, torch.int64, (b, n_words(self.n_sites)), 'packed')
+    if out is None:
+      out = torch.empty(b, ham.n_bonds, dtype=torch.float32, device=packed.device)
+    else:
+      _want(out, torch.float32, (b, ham.n_bonds), 'out')
+    check(load().cgsvmc_bond_values(self._handle, ham._handle, _ptr(packed), b, _ptr(out), _stream()))
+    return out
 
   def weighted_grad_sum(self, packed, weights, out=None):
     self._sync_params()
@@ -595,6 +612,26 @@ def local_energy_from_amps(ham, packed, logabs, sign, flipped_logabs, flipped_si
                                              _ptr(flipped_logabs), _ptr(flipped_sign), _ptr(e),
                                              _ptr(diag), _ptr(off), _stream()))
   return (e, diag, off) if want_parts else e
+
+
+def bond_values_from_amps(ham, packed, logabs, sign, flipped_logabs, flipped_sign, out=None):
+  """float32 [B, n_bonds]: the per-bond terms of local_energy_from_amps
+  (cgsvmc_bond_values_from_amps), for any wavefunction."""
+  b = packed.shape[0]
+  _want(packed, torch.int64, (b, n_words(ham.n_sites)), 'packed')
+  _want(logabs, torch.float32, (b,), 'logabs')
+  _want(flipped_logabs, torch.float32, (b, ham.n_bonds), 'flipped_logabs')
+  if sign is not None:
+    _want(sign, torch.float32, (b,), 'sign')
+  if flipped_sign is not None:
+    _want(flipped_sign, torch.float32, (b, ham.n_bonds), 'flipped_sign')
+  if out is None:
+    out = torch.empty(b, ham.n_bonds, dtype=torch.float32, device=packed.device)
+  else:
+    _want(out, torch.float32, (b, ham.n_bonds), 'out')
+  check(load().cgsvmc_bond_values_from_amps(ham._handle, _ptr(packed), b, _ptr(logabs), _ptr(sign),
+                                            _ptr(flipped_logabs), _ptr(flipped_sign), _ptr(out), _stream()))
+  return out
 
 
 

@@ -398,6 +398,40 @@ int cgsvmc_local_energy(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint6
                           (cudaStream_t)stream);
 }
 
+int cgsvmc_bond_values(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, int64_t B,
+                       float* values, void* stream) {
+  NvtxRange range("cgsvmc:K3 bond_values");
+  if (int rc = check_ready(a)) return rc;
+  if (h == nullptr) return invalid("bond_values: NULL hamiltonian");
+  if (h->n_sites != a->desc.n_sites) return invalid("bond_values: hamiltonian and ansatz n_sites differ");
+  if (B < 0) return invalid("bond_values: n_walkers < 0");
+  // before the empty-batch return, so that a call with no walkers probes for support
+  if (!rbm_fast_supported(a)) {
+    set_error("bond_values: built for the pure RBM only (rbm, no hidden layers, H <= 256, "
+              "1, 2 or 4 spin words); use cgsvmc_bond_values_from_amps");
+    return CGSVMC_ERR_UNSUPPORTED;
+  }
+  if (B == 0) return CGSVMC_OK;
+  if (packed == nullptr) return invalid("bond_values: NULL configs");
+  if (h->n_bonds == 0) return CGSVMC_OK;
+  if (values == nullptr) return invalid("bond_values: NULL buffer");
+  return rbm_bond_values(a, h, packed, B, values, (cudaStream_t)stream);
+}
+
+int cgsvmc_bond_values_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B, const float* logabs,
+                                 const float* sign, const float* flipped_logabs, const float* flipped_sign,
+                                 float* values, void* stream) {
+  NvtxRange range("cgsvmc:K3 bond_values_from_amps");
+  if (h == nullptr) return invalid("bond_values_from_amps: NULL hamiltonian");
+  if (B < 0) return invalid("bond_values_from_amps: n_walkers < 0");
+  if (B == 0) return CGSVMC_OK;
+  if (packed == nullptr || logabs == nullptr) return invalid("bond_values_from_amps: NULL buffer");
+  if (h->n_bonds == 0) return CGSVMC_OK;
+  if (flipped_logabs == nullptr || values == nullptr) return invalid("bond_values_from_amps: NULL buffer");
+  return launch_bond_values_from_amps(h, packed, B, logabs, sign, flipped_logabs, flipped_sign, values,
+                                      (cudaStream_t)stream);
+}
+
 int cgsvmc_weighted_grad_sum(const cgsvmc_ansatz* a, const uint64_t* packed, const float* weights,
                              int64_t B, int32_t K, float* out, void* stream) {
   NvtxRange range("cgsvmc:K4 weighted_grad_sum");

@@ -84,6 +84,9 @@ int launch_accept_exchange(uint64_t* packed, const uint64_t* proposed, int64_t B
 int launch_eloc_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B, const float* logabs,
                           const float* sign, const float* flipped_logabs, const float* flipped_sign,
                           float* e_loc, float* diag, float* off, cudaStream_t s);
+int launch_bond_values_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B, const float* logabs,
+                                 const float* sign, const float* flipped_logabs, const float* flipped_sign,
+                                 float* values, cudaStream_t s);
 int launch_fill(float* dst, int64_t n, float value, cudaStream_t s);
 int launch_energy_stats(const float* e, int64_t B, double* stats, cudaStream_t s);
 int launch_reduce_partials(const float* partials, int n_parts, int64_t n, float* out,
@@ -115,6 +118,9 @@ int rbm_mc_replay(const cgsvmc_ansatz* a, uint64_t* packed, int64_t B, const flo
 int rbm_local_energy(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed,
                      int64_t B, float* e_loc, float* log_amp_out, float* diag_out,
                      float* off_out, cudaStream_t s);
+// values [B, n_bonds]: the per-bond terms of rbm_local_energy (n_bonds >= 1)
+int rbm_bond_values(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, int64_t B,
+                    float* values, cudaStream_t s);
 
 // ---- pure RBM, second generation (rbm2.cu): ratio tables, 4 walkers per warp ----
 // h may be NULL in rbm2_supported (sampler only).

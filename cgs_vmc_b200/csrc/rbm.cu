@@ -13,8 +13,9 @@
 // plans every shape accepted here.  This file keeps what rbm2 does not cover:
 // the amplitudes (log_amp) and their directional derivative (log_amp_jvp, the
 // forward half of the matrix-free S v of stochastic reconfiguration), the one-step replay of the reference's Metropolis
-// step (parity hook), and the local energy of Hamiltonians whose bond staging
-// does not fit rbm2's shared memory (N = 256, H = 144: rbm2 takes at most 200 bonds).
+// step (parity hook), the local energy of Hamiltonians whose bond staging
+// does not fit rbm2's shared memory (N = 256, H = 144: rbm2 takes at most 200 bonds),
+// and the per-bond terms of the local energy (bond values: spin-spin correlations).
 #include "common.cuh"
 #include "internal.h"
 
@@ -308,6 +309,61 @@ rbm_local_energy_kernel(RbmParams p, const int2* __restrict__ bonds_ij,
 }
 
 // ---------------------------------------------------------------------------
+// K3 per bond: values[b, k] = jz_k/4 s_i s_j + jx_k/2 [s_i != s_j] psi(flip_k)/psi,
+// the summands of rbm_local_energy_kernel kept instead of reduced.  Any number
+// of bonds: the first n_staged go to shared memory behind the parameter image,
+// the rest are read through the read-only path (every lane reads the same bond:
+// one broadcast transaction).  Lane k & 31 keeps bond k's value and the warp
+// stores 32 consecutive values at a time.
+// ---------------------------------------------------------------------------
+template <int NW, int KJ, bool WS>
+__global__ void __launch_bounds__(kThreads)
+rbm_bond_values_kernel(RbmParams p, const int2* __restrict__ bonds_ij,
+                       const float* __restrict__ bonds_jx, const float* __restrict__ bonds_jz,
+                       int n_bonds, int n_staged, const uint64_t* __restrict__ packed, int64_t B,
+                       float* __restrict__ values) {
+  extern __shared__ float smem[];
+  const float *a_s, *Wp; int ldw;
+  const int param_floats = round_up(p.N, 32) + (WS ? p.N * 32 * KJ : 0);
+  int4* bond_s = reinterpret_cast<int4*>(smem + round_up(param_floats, 4));
+  for (int k = threadIdx.x; k < n_staged; k += blockDim.x) {
+    const int2 ij = bonds_ij[k];
+    bond_s[k] = make_int4(ij.x, ij.y, __float_as_int(bonds_jx[k]), __float_as_int(bonds_jz[k]));
+  }
+  stage_params<KJ, WS>(p, smem, a_s, Wp, ldw);   // ends with the CTA barrier
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int64_t b = (int64_t)blockIdx.x * kWarps + warp; b < B; b += (int64_t)gridDim.x * kWarps) {
+    uint64_t s[NW]; float th[KJ], lc[KJ];
+    load_spins<NW>(packed, b, s);
+    init_theta<NW, KJ, WS>(p, Wp, ldw, s, lane, th, lc);
+    float* row = values + b * (int64_t)n_bonds;
+    float keep = 0.f;
+    for (int k = 0; k < n_bonds; ++k) {
+      int4 bd;
+      if (k < n_staged) {
+        bd = bond_s[k];
+      } else {
+        const int2 ij = __ldg(bonds_ij + k);
+        bd = make_int4(ij.x, ij.y, __float_as_int(__ldg(bonds_jx + k)), __float_as_int(__ldg(bonds_jz + k)));
+      }
+      const int bi = get_bit<NW>(s, bd.x), bj = get_bit<NW>(s, bd.y);
+      const float jx = __int_as_float(bd.z), jz = __int_as_float(bd.w);
+      float v = (bi == bj ? 0.25f : -0.25f) * jz;
+      if (bi != bj && jx != 0.f) {   // warp-uniform: the spins are replicated in every lane
+        const int up = bi ? bd.x : bd.y, dn = bi ? bd.y : bd.x;
+        float tn[KJ], ln[KJ];
+        const float dl = exchange_log_ratio<KJ, WS>(p, a_s, Wp, ldw, up, dn, lane, th, lc, tn, ln);
+        v += (0.5f * jx) * fast_exp(dl);
+      }
+      if (lane == (k & 31)) keep = v;
+      if ((k & 31) == 31 || k == n_bonds - 1) {
+        if (lane <= (k & 31)) row[(k & ~31) + lane] = keep;
+      }
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------
 // host-side dispatch
 // ---------------------------------------------------------------------------
 // `flat` is a vector in the flat parameter layout: the parameters or a tangent.
@@ -447,6 +503,27 @@ int rbm_local_energy(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t
   RBM_DISPATCH(BODY)
 #undef BODY
   return cuda_fail(cudaGetLastError(), "rbm_local_energy launch");
+}
+
+int rbm_bond_values(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, int64_t B,
+                    float* values, cudaStream_t st) {
+  const RbmParams p = make_params(a);
+  const Geometry g = geometry(a);
+  const int grid = grid_for(a, B);
+  // bonds fill the shared memory beside the parameter image up to 112 KB, which
+  // keeps two CTAs per SM (geometry() caps the image at 96 KB)
+  constexpr size_t kSmemBudget = 112 * 1024;
+  const size_t param_bytes = round_up((int)g.param_bytes, 16);
+  const int n_staged = (int)std::min<size_t>((size_t)h->n_bonds, (kSmemBudget - param_bytes) / sizeof(int4));
+  const size_t smem = param_bytes + (size_t)n_staged * sizeof(int4);
+#define BODY(NWV, KJV, WSV)                                                        \
+  { auto kern = rbm_bond_values_kernel<NWV, KJV, WSV>;                            \
+    if (int rc = set_smem(kern, smem)) return rc;                                 \
+    kern<<<grid, kThreads, smem, st>>>(p, h->ij, h->jx, h->jz, h->n_bonds, n_staged, packed, B, \
+                                       values); }
+  RBM_DISPATCH(BODY)
+#undef BODY
+  return cuda_fail(cudaGetLastError(), "rbm_bond_values launch");
 }
 
 }  // namespace cgsvmc

@@ -256,6 +256,34 @@ __global__ void eloc_from_amps_kernel(const int2* __restrict__ ij, const float* 
   }
 }
 
+// The summands of eloc_from_amps_kernel kept per bond: values[b, k] (same
+// layout as flipped_*); the ratio is not read where jx_k == 0.
+__global__ void bond_values_from_amps_kernel(const int2* __restrict__ ij, const float* __restrict__ jx,
+                                             const float* __restrict__ jz, int n_bonds,
+                                             const uint64_t* __restrict__ packed, int64_t B, int W,
+                                             const float* __restrict__ logabs, const float* __restrict__ sign,
+                                             const float* __restrict__ flipped_logabs,
+                                             const float* __restrict__ flipped_sign, float* __restrict__ values) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t b = warp; b < B; b += n_warps) {
+    const float la = logabs[b], sg = sign != nullptr ? sign[b] : 1.f;
+    for (int k = lane; k < n_bonds; k += 32) {
+      const int2 bd = ij[k];
+      const uint64_t wi = packed[b * W + (bd.x >> 6)], wj = packed[b * W + (bd.y >> 6)];
+      const bool anti = (((wi >> (bd.x & 63)) ^ (wj >> (bd.y & 63))) & 1ull) != 0;
+      const int64_t e = b * n_bonds + k;
+      float v = (anti ? -0.25f : 0.25f) * jz[k];
+      if (anti && jx[k] != 0.f) {
+        const float sf = flipped_sign != nullptr ? flipped_sign[e] : 1.f;
+        v += 0.5f * jx[k] * sf * sg * expf(flipped_logabs[e] - la);
+      }
+      values[e] = v;
+    }
+  }
+}
+
 // SupervisedWavefunctionOptimizer (training.py:166-175): per walker
 //   r_b = sign sign_t exp(z_t + log_norm - z)   (= psi_target sqrt(2^N) / psi)
 //   loss  += sum_b (1 - r_b)^2                  (mean_b (psi - t)^2 / sg(psi)^2 times the batch size)
@@ -553,6 +581,16 @@ int launch_eloc_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B
       h->ij, h->jx, h->jz, h->n_bonds, packed, B, n_words(h->n_sites), logabs, sign, flipped_logabs,
       flipped_sign, e_loc, diag, off);
   return cuda_fail(cudaGetLastError(), "eloc_from_amps launch");
+}
+
+int launch_bond_values_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B, const float* logabs,
+                                 const float* sign, const float* flipped_logabs, const float* flipped_sign,
+                                 float* values, cudaStream_t s) {
+  if (B == 0 || h->n_bonds == 0) return CGSVMC_OK;
+  bond_values_from_amps_kernel<<<blocks_for(B, kThreads / 32), kThreads, 0, s>>>(
+      h->ij, h->jx, h->jz, h->n_bonds, packed, B, n_words(h->n_sites), logabs, sign, flipped_logabs,
+      flipped_sign, values);
+  return cuda_fail(cudaGetLastError(), "bond_values_from_amps launch");
 }
 
 }  // namespace cgsvmc

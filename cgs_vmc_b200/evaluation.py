@@ -22,7 +22,9 @@ class MonteCarloOperatorEvaluator(WavefunctionEvaluator):
   """Operator evaluation by MCMC."""
 
   def build_eval_ops(self, wavefunction, operator, hparams, shared_resources):
-    """evaluation.py:77-110: value = mean of the local values."""
+    """evaluation.py:77-110: value = mean of the local values.  An operator
+    with a vector local value [B, K] (operators.HeisenbergBonds) gives the
+    float64 numpy vector [K] of the per-column means."""
     n_sites = hparams.num_sites
     local_batch, walker_id0 = distributed.shard(hparams.batch_size)
     configs = graph_builders.get_configs(shared_resources, local_batch, n_sites,
@@ -32,6 +34,9 @@ class MonteCarloOperatorEvaluator(WavefunctionEvaluator):
 
     def value():
       e = operator.local_value(wavefunction, configs)
+      if e.dim() == 2:
+        totals = distributed.allreduce_(e.double().sum(dim=0))
+        return totals.cpu().numpy() / hparams.batch_size
       total = distributed.allreduce_(e.double().sum())
       return float(total.item()) / hparams.batch_size
 

@@ -24,6 +24,10 @@ class Operator:
     raise NotImplementedError
 
 
+# values per chunk of walkers in _BondListOperator.bond_values (128 MB of float32)
+_BOND_VALUES_CHUNK = 1 << 25
+
+
 class _BondListOperator(Operator):
   def __init__(self, bonds, j_x, j_z):
     self._bonds_list = [(int(a), int(b)) for a, b in bonds]
@@ -64,6 +68,45 @@ class _BondListOperator(Operator):
         fs.float().reshape(b, ham.n_bonds).contiguous(), want_parts=True)
     return e, logabs, sign, diag, off
 
+  def bond_values(self, wavefunction, inputs):
+    """float32 [B, n_bonds]: each bond's term of the local value,
+    jz/4 s_i s_j + jx/2 [s_i != s_j] psi(flipped) / psi.  A single pure RBM
+    runs the fused kernel; every other wavefunction goes through psi on the
+    bond-flipped configurations, like _evaluate.  Walkers are processed in
+    chunks of at most _BOND_VALUES_CHUNK values (the flipped configurations of
+    the amplitude route scale with it too)."""
+    from . import graph_builders
+    n = inputs.shape[1]
+    packed = graph_builders.as_packed(inputs, n)
+    ham = self.native(n)
+    b, k = packed.shape[0], ham.n_bonds
+    out = torch.empty(b, k, dtype=torch.float32, device=packed.device)
+    if b == 0 or k == 0:
+      return out
+    fused = None
+    if wavefunction.fast_path:
+      fused = wavefunction.native(n)
+      try:
+        fused.bond_values(ham, packed[:0])        # no walkers: probes for support
+      except NotImplementedError:
+        fused = None
+    else:
+      wavefunction.connect(n)
+    chunk = max(1, _BOND_VALUES_CHUNK // k)
+    for c0 in range(0, b, chunk):
+      pc, oc = packed[c0:c0 + chunk], out[c0:c0 + chunk]
+      if fused is not None:
+        fused.bond_values(ham, pc, out=oc)
+        continue
+      bc = pc.shape[0]
+      logabs, sign = wavefunction.amplitudes(pc)
+      _, flipped = ham.flip_enum(pc, want_flipped=True)
+      fl, fs = wavefunction.amplitudes(flipped.reshape(bc * k, -1))
+      _native.bond_values_from_amps(
+          ham, pc, logabs.float().contiguous(), sign.float().contiguous(),
+          fl.float().reshape(bc, k).contiguous(), fs.float().reshape(bc, k).contiguous(), out=oc)
+    return out
+
   def build(self, wavefunction, inputs, psi=None):
     """(diagonal matrix element, off-diagonal term) of <R|O|psi>
     (operators.py:137-169, 227-247)."""
@@ -98,3 +141,20 @@ class HeisenbergHamiltonian(_BondListOperator):
   def __init__(self, bonds, j_x, j_z):
     super().__init__(bonds, j_x, j_z)
     self._heisenberg_bonds = self._bonds_list
+
+
+class HeisenbergBonds(_BondListOperator):
+  """Many HeisenbergBond at once: the local value is the vector of the bonds'
+  local values, float32 [B, n_bonds], from one pass over the walkers.  With
+  site pairs and j_x = j_z = 1 these are the spin-spin correlations
+  S_i . S_j (lattices.all_pairs; in a Marshall-rotated frame j_x = sign_i
+  sign_j, lattices.marshall_signs)."""
+
+  def local_value(self, wavefunction, inputs, psi=None):
+    return self.bond_values(wavefunction, inputs)
+
+  def build(self, wavefunction, inputs, psi=None):
+    raise NotImplementedError('HeisenbergBonds has a vector local value only')
+
+  def apply_in_place(self, wavefunction, inputs, psi=None):
+    raise NotImplementedError('HeisenbergBonds has a vector local value only')

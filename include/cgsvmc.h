@@ -234,6 +234,19 @@ int cgsvmc_local_energy(const cgsvmc_ansatz* ansatz, const cgsvmc_ham* ham,
                         float* e_loc, float* log_amp_out, float* diag_out,
                         float* offdiag_ratio_out, void* stream);
 
+/* The terms of cgsvmc_local_energy kept per bond instead of summed:
+ *   values[b, k] = jz_k/4 s_i s_j + jx_k/2 [s_i != s_j] psi(flip_k)/psi
+ * (float32 [B, n_bonds], row-major), so sum_k values[b, k] = e_loc[b] up to
+ * float32 summation order.  The ratio is not evaluated where jx_k == 0.  With a
+ * bond list of site pairs and jx = jz = 1, values[b, k] is the local value of
+ * S_i . S_j: one pass over the walkers gives every spin-spin correlation.
+ * Built for the pure RBM (the shapes of cgsvmc_log_amp_jvp); any other ansatz
+ * returns CGSVMC_ERR_UNSUPPORTED, also with n_walkers == 0, so a call without
+ * walkers probes for support.  Any number of bonds. */
+int cgsvmc_bond_values(const cgsvmc_ansatz* ansatz, const cgsvmc_ham* ham,
+                       const uint64_t* packed, int64_t n_walkers, float* values,
+                       void* stream);
+
 /* ---- estimators ------------------------------------------------------- */
 
 /* Replaces the two tf.gradients + accumulators of
@@ -389,6 +402,14 @@ int cgsvmc_local_energy_from_amps(const cgsvmc_ham* ham, const uint64_t* packed,
                                   const float* flipped_sign, float* e_loc,
                                   float* diag_out, float* offdiag_ratio_out,
                                   void* stream);
+/* The per-bond form of cgsvmc_local_energy_from_amps (same arguments): values
+ * float32 [B, n_bonds] as in cgsvmc_bond_values, for every ansatz (signed
+ * outputs and composites too).  The ratio is not read where jx_k == 0. */
+int cgsvmc_bond_values_from_amps(const cgsvmc_ham* ham, const uint64_t* packed,
+                                 int64_t n_walkers, const float* logabs,
+                                 const float* sign, const float* flipped_logabs,
+                                 const float* flipped_sign, float* values,
+                                 void* stream);
 
 /* Replaces tf.metrics.mean(local_energy) bookkeeping (training.py:555):
  * stats (double [4], device) += { sum e, sum e^2, B, 0 }. */

@@ -10,13 +10,16 @@ from absl import flags
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
-from cgs_vmc_b200 import checkpoint, drivers, evaluation, operators, utils, wavefunctions  # noqa: E402
+from cgs_vmc_b200 import checkpoint, drivers, evaluation, lattices, operators, utils, wavefunctions  # noqa: E402
 from cgs_vmc_b200.session import Session  # noqa: E402
 
 flags.DEFINE_float('heisenberg_jx', 1.0, 'Jx value in Heisenberg Hamiltonian.')
 flags.DEFINE_string('checkpoint_dir', '', 'Full path to the checkpoint directory.')
 flags.DEFINE_string('output_file', '', 'Optional file for the result.')
 flags.DEFINE_string('hparams', '', 'Comma-separated name=value overrides.')
+flags.DEFINE_string('correlations_file', '',
+                    'Optional .npz for the spin-spin correlations <S_i . S_j> of all site pairs '
+                    '(and the structure factor when the lattice geometry is known).')
 FLAGS = flags.FLAGS
 
 
@@ -28,6 +31,8 @@ def main(argv):
   bonds, j_x, j_z = drivers.load_bonds(FLAGS.checkpoint_dir, hparams.num_sites, FLAGS.heisenberg_jx)
   wavefunction = wavefunctions.build_wavefunction(hparams)
   hamiltonian = operators.HeisenbergHamiltonian(bonds, j_x, j_z)
+  # before the energy run: a bond set without Marshall signs fails early
+  signs = lattices.marshall_signs(hparams.num_sites, bonds, j_x, j_z) if FLAGS.correlations_file else None
   evaluator = evaluation.MonteCarloOperatorEvaluator()
   shared_resources = {}
   evaluation_ops = evaluator.build_eval_ops(
@@ -49,6 +54,39 @@ def main(argv):
       with open(FLAGS.output_file, 'w') as f:
         f.write('Energy mean: {}\nUncertainty: {}\nStderr: {}\n'.format(
             mean_energy, reference_uncertainty, stderr))
+  if FLAGS.correlations_file:
+    evaluate_correlations(evaluator, wavefunction, hparams, shared_resources, session, signs,
+                          has_bond_file=os.path.exists(os.path.join(FLAGS.checkpoint_dir, 'J.txt')),
+                          rank=rank)
+
+
+def evaluate_correlations(evaluator, wavefunction, hparams, shared_resources, session, signs, has_bond_file,
+                          rank):
+  """<S_i . S_j> of every site pair from a second evaluation on the same
+  walkers, in the frame the Hamiltonian was written in (Marshall signs)."""
+  n = hparams.num_sites
+  pairs = np.asarray(lattices.all_pairs(n), dtype=np.int32)
+  jx = (signs[pairs[:, 0]] * signs[pairs[:, 1]]).astype(np.float32)
+  correlations = operators.HeisenbergBonds(pairs, jx, 1.0)
+  ops = evaluator.build_eval_ops(wavefunction=wavefunction, operator=correlations, hparams=hparams,
+                                 shared_resources=shared_resources)
+  samples = np.asarray(evaluator.run_evaluation(ops, session, hparams, epoch_num=0))
+  if rank != 0:
+    return
+  mean = samples.mean(axis=0)
+  stderr = samples.std(axis=0) / np.sqrt(len(samples))
+  matrix = np.full((n, n), 0.75)
+  matrix[pairs[:, 0], pairs[:, 1]] = mean
+  matrix[pairs[:, 1], pairs[:, 0]] = mean
+  out = dict(pairs=pairs, signs=signs, mean=mean, stderr=stderr, matrix=matrix)
+  # geometry: the default bonds are a periodic chain; a bond file is read as
+  # the size_x x size_y square lattice when the sizes match, else S(q) is left out
+  if not has_bond_file:
+    out['structure_factor'] = lattices.structure_factor(matrix, n, 1)
+  elif hparams.size_x * hparams.size_y == n:
+    out['structure_factor'] = lattices.structure_factor(matrix, hparams.size_x, hparams.size_y)
+  with open(FLAGS.correlations_file, 'wb') as f:
+    np.savez(f, **out)
 
 
 if __name__ == '__main__':
