@@ -34,6 +34,7 @@ EXPORTS = [
     'cgsvmc_epoch_end', 'cgsvmc_pack_configs_host', 'cgsvmc_upload_configs',
     'cgsvmc_conv_periodic', 'cgsvmc_log_amp_jvp', 'cgsvmc_rbm2_plan',
     'cgsvmc_bond_values', 'cgsvmc_bond_values_from_amps',
+    'cgsvmc_swap_values', 'cgsvmc_swap_configs', 'cgsvmc_swap_values_from_amps',
 ]
 # cgsvmc_rbm2_plan: entry points (modes) and the fields it reports, in order
 RBM2_PLAN_MODES = {'mc_steps': 0, 'local_energy': 1, 'weighted_grad_sum': 2, 'accumulate': 3,
@@ -97,6 +98,9 @@ def load():
   lib.cgsvmc_local_energy_from_amps.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp]
   lib.cgsvmc_bond_values.argtypes = [vp, vp, vp, i64, vp, vp]
   lib.cgsvmc_bond_values_from_amps.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, vp]
+  lib.cgsvmc_swap_values.argtypes = [vp, vp, i64, vp, i32, vp, vp]
+  lib.cgsvmc_swap_configs.argtypes = [vp, i64, i32, vp, i32, vp, vp]
+  lib.cgsvmc_swap_values_from_amps.argtypes = [vp, i64, i32, vp, i32, vp, vp, vp, vp, vp, vp]
   f32 = ctypes.c_float
   lib.cgsvmc_batch_steps.argtypes = [vp, vp, vp, i64, i32, vp, vp, vp, vp, i32, u64, u64, u64, vp, vp, vp]
   lib.cgsvmc_batch_step_fed.argtypes = [vp, vp, vp, vp, i64, vp, vp, vp, vp, i32, u64, u64, u64, vp, vp, vp, vp]
@@ -283,6 +287,23 @@ class Ansatz:
     else:
       _want(out, torch.float32, (b, ham.n_bonds), 'out')
     check(load().cgsvmc_bond_values(self._handle, ham._handle, _ptr(packed), b, _ptr(out), _stream()))
+    return out
+
+  def swap_values(self, packed, regions, out=None):
+    """float32 [P, R]: the replica-swap values of the pairs (row p, row P + p)
+    of packed [2P, W] over the region masks regions (int64-viewed uint64
+    [R, W]) (cgsvmc_swap_values; pure RBM only, NotImplementedError otherwise
+    -- a call with no pairs probes for support)."""
+    self._sync_params()
+    w = n_words(self.n_sites)
+    p = _pair_count(packed, w)
+    r = regions.shape[0]
+    _want(regions, torch.int64, (r, w), 'regions')
+    if out is None:
+      out = torch.empty(p, r, dtype=torch.float32, device=packed.device)
+    else:
+      _want(out, torch.float32, (p, r), 'out')
+    check(load().cgsvmc_swap_values(self._handle, _ptr(packed), p, _ptr(regions), r, _ptr(out), _stream()))
     return out
 
   def weighted_grad_sum(self, packed, weights, out=None):
@@ -631,6 +652,54 @@ def bond_values_from_amps(ham, packed, logabs, sign, flipped_logabs, flipped_sig
     _want(out, torch.float32, (b, ham.n_bonds), 'out')
   check(load().cgsvmc_bond_values_from_amps(ham._handle, _ptr(packed), b, _ptr(logabs), _ptr(sign),
                                             _ptr(flipped_logabs), _ptr(flipped_sign), _ptr(out), _stream()))
+  return out
+
+
+def _pair_count(packed, w):
+  """P for packed [2P, W] (int64-viewed uint64)."""
+  b = packed.shape[0]
+  _want(packed, torch.int64, (b, w), 'packed')
+  if b % 2:
+    raise ValueError('packed must hold 2 * n_pairs walkers, got %d' % b)
+  return b // 2
+
+
+def swap_configs(packed, n_sites, regions, out=None):
+  """int64-viewed uint64 [P, R, 2, W]: the swapped pairs (sigma1', sigma2') of
+  the pairs (row p, row P + p) of packed [2P, W] over regions [R, W]
+  (cgsvmc_swap_configs)."""
+  w = n_words(n_sites)
+  p = _pair_count(packed, w)
+  r = regions.shape[0]
+  _want(regions, torch.int64, (r, w), 'regions')
+  if out is None:
+    out = torch.empty(p, r, 2, w, dtype=torch.int64, device=packed.device)
+  else:
+    _want(out, torch.int64, (p, r, 2, w), 'out')
+  check(load().cgsvmc_swap_configs(_ptr(packed), p, n_sites, _ptr(regions), r, _ptr(out), _stream()))
+  return out
+
+
+def swap_values_from_amps(packed, n_sites, regions, logabs, sign, swapped_logabs, swapped_sign, out=None):
+  """float32 [P, R]: the replica-swap values from the amplitudes of the pairs
+  (logabs / sign [2P]) and of swap_configs (swapped_* [P, R, 2])
+  (cgsvmc_swap_values_from_amps), for any wavefunction."""
+  w = n_words(n_sites)
+  p = _pair_count(packed, w)
+  r = regions.shape[0]
+  _want(regions, torch.int64, (r, w), 'regions')
+  _want(logabs, torch.float32, (2 * p,), 'logabs')
+  _want(swapped_logabs, torch.float32, (p, r, 2), 'swapped_logabs')
+  if sign is not None:
+    _want(sign, torch.float32, (2 * p,), 'sign')
+  if swapped_sign is not None:
+    _want(swapped_sign, torch.float32, (p, r, 2), 'swapped_sign')
+  if out is None:
+    out = torch.empty(p, r, dtype=torch.float32, device=packed.device)
+  else:
+    _want(out, torch.float32, (p, r), 'out')
+  check(load().cgsvmc_swap_values_from_amps(_ptr(packed), p, n_sites, _ptr(regions), r, _ptr(logabs), _ptr(sign),
+                                            _ptr(swapped_logabs), _ptr(swapped_sign), _ptr(out), _stream()))
   return out
 
 

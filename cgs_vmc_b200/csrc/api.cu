@@ -432,6 +432,56 @@ int cgsvmc_bond_values_from_amps(const cgsvmc_ham* h, const uint64_t* packed, in
                                       (cudaStream_t)stream);
 }
 
+int cgsvmc_swap_values(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t n_pairs, const uint64_t* regions,
+                       int32_t n_regions, float* values, void* stream) {
+  NvtxRange range("cgsvmc:K3 swap_values");
+  if (int rc = check_ready(a)) return rc;
+  if (n_pairs < 0) return invalid("swap_values: n_pairs < 0");
+  if (n_regions < 0) return invalid("swap_values: n_regions < 0");
+  // before the empty-batch return, so that a call with no pairs probes for support
+  if (!rbm_fast_supported(a)) {
+    set_error("swap_values: built for the pure RBM only (rbm, no hidden layers, H <= 256, "
+              "1, 2 or 4 spin words); use cgsvmc_swap_configs and cgsvmc_swap_values_from_amps");
+    return CGSVMC_ERR_UNSUPPORTED;
+  }
+  if (n_pairs == 0) return CGSVMC_OK;
+  if (packed == nullptr) return invalid("swap_values: NULL configs");
+  if (n_regions == 0) return CGSVMC_OK;
+  if (regions == nullptr || values == nullptr) return invalid("swap_values: NULL buffer");
+  return rbm_swap_values(a, packed, n_pairs, regions, n_regions, values, (cudaStream_t)stream);
+}
+
+int cgsvmc_swap_configs(const uint64_t* packed, int64_t n_pairs, int32_t n_sites, const uint64_t* regions,
+                        int32_t n_regions, uint64_t* swapped, void* stream) {
+  NvtxRange range("cgsvmc:K3 swap_configs");
+  if (n_pairs < 0) return invalid("swap_configs: n_pairs < 0");
+  if (n_regions < 0) return invalid("swap_configs: n_regions < 0");
+  if (n_sites < 2 || n_sites > CGSVMC_MAX_SITES) return invalid("swap_configs: n_sites must be in [2, 256]");
+  if (n_pairs == 0) return CGSVMC_OK;
+  if (packed == nullptr) return invalid("swap_configs: NULL configs");
+  if (n_regions == 0) return CGSVMC_OK;
+  if (regions == nullptr || swapped == nullptr) return invalid("swap_configs: NULL buffer");
+  return launch_swap_configs(packed, n_pairs, n_sites, regions, n_regions, swapped, (cudaStream_t)stream);
+}
+
+int cgsvmc_swap_values_from_amps(const uint64_t* packed, int64_t n_pairs, int32_t n_sites, const uint64_t* regions,
+                                 int32_t n_regions, const float* logabs, const float* sign,
+                                 const float* swapped_logabs, const float* swapped_sign, float* values,
+                                 void* stream) {
+  NvtxRange range("cgsvmc:K3 swap_values_from_amps");
+  if (n_pairs < 0) return invalid("swap_values_from_amps: n_pairs < 0");
+  if (n_regions < 0) return invalid("swap_values_from_amps: n_regions < 0");
+  if (n_sites < 2 || n_sites > CGSVMC_MAX_SITES)
+    return invalid("swap_values_from_amps: n_sites must be in [2, 256]");
+  if (n_pairs == 0) return CGSVMC_OK;
+  if (packed == nullptr || logabs == nullptr) return invalid("swap_values_from_amps: NULL buffer");
+  if (n_regions == 0) return CGSVMC_OK;
+  if (regions == nullptr || swapped_logabs == nullptr || values == nullptr)
+    return invalid("swap_values_from_amps: NULL buffer");
+  return launch_swap_values_from_amps(packed, n_pairs, n_sites, regions, n_regions, logabs, sign, swapped_logabs,
+                                      swapped_sign, values, (cudaStream_t)stream);
+}
+
 int cgsvmc_weighted_grad_sum(const cgsvmc_ansatz* a, const uint64_t* packed, const float* weights,
                              int64_t B, int32_t K, float* out, void* stream) {
   NvtxRange range("cgsvmc:K4 weighted_grad_sum");

@@ -87,6 +87,13 @@ int launch_eloc_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B
 int launch_bond_values_from_amps(const cgsvmc_ham* h, const uint64_t* packed, int64_t B, const float* logabs,
                                  const float* sign, const float* flipped_logabs, const float* flipped_sign,
                                  float* values, cudaStream_t s);
+// replica swap: pairs are rows (p, P + p) of packed [2P, W]; regions uint64 [R, W]
+int launch_swap_configs(const uint64_t* packed, int64_t P, int N, const uint64_t* regions, int n_regions,
+                        uint64_t* swapped, cudaStream_t s);
+int launch_swap_values_from_amps(const uint64_t* packed, int64_t P, int N, const uint64_t* regions,
+                                 int n_regions, const float* logabs, const float* sign,
+                                 const float* swapped_logabs, const float* swapped_sign, float* values,
+                                 cudaStream_t s);
 int launch_fill(float* dst, int64_t n, float value, cudaStream_t s);
 int launch_energy_stats(const float* e, int64_t B, double* stats, cudaStream_t s);
 int launch_reduce_partials(const float* partials, int n_parts, int64_t n, float* out,
@@ -121,6 +128,9 @@ int rbm_local_energy(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t
 // values [B, n_bonds]: the per-bond terms of rbm_local_energy (n_bonds >= 1)
 int rbm_bond_values(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t* packed, int64_t B,
                     float* values, cudaStream_t s);
+// values [P, n_regions]: the replica-swap values of pairs (p, P + p) (n_regions >= 1)
+int rbm_swap_values(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t P, const uint64_t* regions,
+                    int n_regions, float* values, cudaStream_t s);
 
 // ---- pure RBM, second generation (rbm2.cu): ratio tables, 4 walkers per warp ----
 // h may be NULL in rbm2_supported (sampler only).

@@ -15,7 +15,8 @@
 // forward half of the matrix-free S v of stochastic reconfiguration), the one-step replay of the reference's Metropolis
 // step (parity hook), the local energy of Hamiltonians whose bond staging
 // does not fit rbm2's shared memory (N = 256, H = 144: rbm2 takes at most 200 bonds),
-// and the per-bond terms of the local energy (bond values: spin-spin correlations).
+// the per-bond terms of the local energy (bond values: spin-spin correlations),
+// and the replica-swap values of the second Renyi entropy.
 #include "common.cuh"
 #include "internal.h"
 
@@ -364,6 +365,119 @@ rbm_bond_values_kernel(RbmParams p, const int2* __restrict__ bonds_ij,
 }
 
 // ---------------------------------------------------------------------------
+// Replica swap (second Renyi entropy): pair p = (sigma1 = row p, sigma2 = row
+// P + p); for region A (mask & valid sites) and D = (sigma1 ^ sigma2) & A,
+//   values[p, r] = psi(sigma1 ^ D) psi(sigma2 ^ D) / (psi(sigma1) psi(sigma2))
+// with 0 when the replicas hold different numbers of up spins in A (the
+// swapped pair leaves the sampled S^z sector) and exactly 1 when D is empty
+// or holds every differing site (the swapped pair is the pair itself).  The
+// visible bias cancels; with Delta_j = sum_{i in D} s2_i W_ij
+//   log r = sum_j lc(th1_j + 2 Delta_j) - lc1_j + lc(th2_j - 2 Delta_j) - lc2_j.
+// Delta is summed over D in increasing site order: it extends the last
+// computed region's Delta when that D is a prefix of this one (nested
+// prefixes: O(N H) per pair for the whole list) and restarts from 0
+// otherwise, the same float32 additions either way, so a region's value does
+// not depend on the list around it.  Lane r & 31 keeps region r's value and
+// the warp stores 32 consecutive values at a time.
+// ---------------------------------------------------------------------------
+template <int NW, int KJ, bool WS>
+__global__ void __launch_bounds__(kThreads)
+rbm_swap_values_kernel(RbmParams p, const uint64_t* __restrict__ packed, int64_t P,
+                       const uint64_t* __restrict__ regions, int n_regions, float* __restrict__ values) {
+  extern __shared__ float smem[];
+  const float *a_s, *Wp; int ldw;
+  stage_params<KJ, WS>(p, smem, a_s, Wp, ldw);   // ends with the CTA barrier
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int64_t b = (int64_t)blockIdx.x * kWarps + warp; b < P; b += (int64_t)gridDim.x * kWarps) {
+    uint64_t s1[NW], s2[NW], dprev[NW];
+    float th1[KJ], lc1[KJ], th2[KJ], lc2[KJ], dl[KJ];
+    load_spins<NW>(packed, b, s1);
+    load_spins<NW>(packed, P + b, s2);
+    init_theta<NW, KJ, WS>(p, Wp, ldw, s1, lane, th1, lc1);
+    init_theta<NW, KJ, WS>(p, Wp, ldw, s2, lane, th2, lc2);
+#pragma unroll
+    for (int w = 0; w < NW; ++w) dprev[w] = 0ull;
+#pragma unroll
+    for (int k = 0; k < KJ; ++k) dl[k] = 0.f;
+    float* row = values + b * (int64_t)n_regions;
+    float keep = 0.f;
+    for (int r = 0; r < n_regions; ++r) {
+      uint64_t d[NW];
+      int up1 = 0, up2 = 0;
+      bool empty = true, whole = true;
+#pragma unroll
+      for (int w = 0; w < NW; ++w) {
+        const uint64_t valid = valid_mask_word(p.N, w);
+        const uint64_t m = __ldg(regions + (int64_t)r * NW + w) & valid;
+        const uint64_t diff = s1[w] ^ s2[w];
+        d[w] = diff & m;
+        up1 += __popcll(s1[w] & m);
+        up2 += __popcll(s2[w] & m);
+        empty = empty && d[w] == 0ull;
+        whole = whole && d[w] == (diff & valid);
+      }
+      float v;
+      if (up1 != up2) {
+        v = 0.f;
+      } else if (empty || whole) {
+        v = 1.f;
+      } else {
+        // extend iff D restricted to the sites up to dprev's highest one is dprev
+        bool extend = true;
+        bool below = false;   // word w lies below dprev's highest non-zero word
+#pragma unroll
+        for (int w = NW - 1; w >= 0; --w) {
+          uint64_t upto;
+          if (below) {
+            upto = ~0ull;
+          } else if (dprev[w] != 0ull) {
+            const int hb = 63 - __clzll(dprev[w]);
+            upto = hb == 63 ? ~0ull : (2ull << hb) - 1ull;
+            below = true;
+          } else {
+            upto = 0ull;
+          }
+          extend = extend && (d[w] & upto) == dprev[w];
+        }
+        if (!extend) {
+#pragma unroll
+          for (int k = 0; k < KJ; ++k) dl[k] = 0.f;
+#pragma unroll
+          for (int w = 0; w < NW; ++w) dprev[w] = 0ull;
+        }
+#pragma unroll
+        for (int w = 0; w < NW; ++w) {
+          uint64_t add = d[w] & ~dprev[w];   // new sites of this word, in increasing order
+          while (add != 0ull) {
+            const int bpos = __ffsll((long long)add) - 1;
+            add &= add - 1ull;
+            const uint32_t flip = (uint32_t)(((s2[w] >> bpos) & 1ull) ^ 1ull) << 31;
+            const float* wrow = Wp + (size_t)(64 * w + bpos) * ldw;
+#pragma unroll
+            for (int k = 0; k < KJ; ++k) {
+              const int j = lane + 32 * k;
+              if (WS || j < p.H) dl[k] += __uint_as_float(__float_as_uint(wrow[j]) ^ flip);
+            }
+          }
+          dprev[w] = d[w];
+        }
+        float part = 0.f;
+#pragma unroll
+        for (int k = 0; k < KJ; ++k) {
+          part += log_cosh(fmaf(2.f, dl[k], th1[k])) - lc1[k];
+          part += log_cosh(fmaf(-2.f, dl[k], th2[k])) - lc2[k];
+        }
+        v = fast_exp(warp_sum(part));
+      }
+      if (lane == (r & 31)) keep = v;
+      if ((r & 31) == 31 || r == n_regions - 1) {
+        if (lane <= (r & 31)) row[(r & ~31) + lane] = keep;
+      }
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------
 // host-side dispatch
 // ---------------------------------------------------------------------------
 // `flat` is a vector in the flat parameter layout: the parameters or a tangent.
@@ -524,6 +638,21 @@ int rbm_bond_values(const cgsvmc_ansatz* a, const cgsvmc_ham* h, const uint64_t*
   RBM_DISPATCH(BODY)
 #undef BODY
   return cuda_fail(cudaGetLastError(), "rbm_bond_values launch");
+}
+
+int rbm_swap_values(const cgsvmc_ansatz* a, const uint64_t* packed, int64_t P, const uint64_t* regions,
+                    int n_regions, float* values, cudaStream_t st) {
+  const RbmParams p = make_params(a);
+  const Geometry g = geometry(a);
+  const int grid = grid_for(a, P);
+  const size_t smem = g.param_bytes;
+#define BODY(NWV, KJV, WSV)                                                        \
+  { auto kern = rbm_swap_values_kernel<NWV, KJV, WSV>;                            \
+    if (int rc = set_smem(kern, smem)) return rc;                                 \
+    kern<<<grid, kThreads, smem, st>>>(p, packed, P, regions, n_regions, values); }
+  RBM_DISPATCH(BODY)
+#undef BODY
+  return cuda_fail(cudaGetLastError(), "rbm_swap_values launch");
 }
 
 }  // namespace cgsvmc

@@ -284,6 +284,68 @@ __global__ void bond_values_from_amps_kernel(const int2* __restrict__ ij, const 
   }
 }
 
+// Replica swap, one thread per (pair, region): sigma1 = row p, sigma2 = row
+// P + p, D = (sigma1 ^ sigma2) & region & valid sites.  swapped[p, r] =
+// (sigma1 ^ D, sigma2 ^ D), uint64 [P, R, 2, W].
+__global__ void swap_configs_kernel(const uint64_t* __restrict__ packed, int64_t P, int N, int W,
+                                    const uint64_t* __restrict__ regions, int n_regions,
+                                    uint64_t* __restrict__ swapped) {
+  const int64_t total = P * n_regions;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total;
+       e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t p = e / n_regions;
+    const int r = (int)(e - p * n_regions);
+    for (int w = 0; w < W; ++w) {
+      const uint64_t s1 = packed[p * W + w], s2 = packed[(P + p) * W + w];
+      const uint64_t d = (s1 ^ s2) & regions[(int64_t)r * W + w] & valid_mask_word(N, w);
+      swapped[(e * 2) * W + w] = s1 ^ d;
+      swapped[(e * 2 + 1) * W + w] = s2 ^ d;
+    }
+  }
+}
+
+// values[p, r] from the amplitudes of the pair (logabs / sign [2P]) and of the
+// swapped pair of swap_configs_kernel (swapped_* [P, R, 2]): 0 when the
+// replicas hold different numbers of up spins in the region, exactly 1 when D
+// is empty or holds every differing site, else
+// sign products * exp((l1' - l1) + (l2' - l2)).  Sign arrays may be NULL (+1).
+__global__ void swap_values_from_amps_kernel(const uint64_t* __restrict__ packed, int64_t P, int N, int W,
+                                             const uint64_t* __restrict__ regions, int n_regions,
+                                             const float* __restrict__ logabs, const float* __restrict__ sign,
+                                             const float* __restrict__ swapped_logabs,
+                                             const float* __restrict__ swapped_sign, float* __restrict__ values) {
+  const int64_t total = P * n_regions;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total;
+       e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t p = e / n_regions;
+    const int r = (int)(e - p * n_regions);
+    int up1 = 0, up2 = 0;
+    bool empty = true, whole = true;
+    for (int w = 0; w < W; ++w) {
+      const uint64_t valid = valid_mask_word(N, w);
+      const uint64_t s1 = packed[p * W + w], s2 = packed[(P + p) * W + w];
+      const uint64_t m = regions[(int64_t)r * W + w] & valid;
+      const uint64_t diff = s1 ^ s2, d = diff & m;
+      up1 += __popcll(s1 & m);
+      up2 += __popcll(s2 & m);
+      empty = empty && d == 0ull;
+      whole = whole && d == (diff & valid);
+    }
+    float v;
+    if (up1 != up2) {
+      v = 0.f;
+    } else if (empty || whole) {
+      v = 1.f;
+    } else {
+      float sg = 1.f;
+      if (sign != nullptr) sg = sign[p] * sign[P + p];
+      if (swapped_sign != nullptr) sg *= swapped_sign[2 * e] * swapped_sign[2 * e + 1];
+      v = sg * expf((swapped_logabs[2 * e] - logabs[p]) + (swapped_logabs[2 * e + 1] - logabs[P + p]));
+    }
+    values[e] = v;
+  }
+}
+
 // SupervisedWavefunctionOptimizer (training.py:166-175): per walker
 //   r_b = sign sign_t exp(z_t + log_norm - z)   (= psi_target sqrt(2^N) / psi)
 //   loss  += sum_b (1 - r_b)^2                  (mean_b (psi - t)^2 / sg(psi)^2 times the batch size)
@@ -591,6 +653,24 @@ int launch_bond_values_from_amps(const cgsvmc_ham* h, const uint64_t* packed, in
       h->ij, h->jx, h->jz, h->n_bonds, packed, B, n_words(h->n_sites), logabs, sign, flipped_logabs,
       flipped_sign, values);
   return cuda_fail(cudaGetLastError(), "bond_values_from_amps launch");
+}
+
+int launch_swap_configs(const uint64_t* packed, int64_t P, int N, const uint64_t* regions, int n_regions,
+                        uint64_t* swapped, cudaStream_t s) {
+  if (P == 0 || n_regions == 0) return CGSVMC_OK;
+  swap_configs_kernel<<<blocks_for(P * n_regions, kThreads), kThreads, 0, s>>>(
+      packed, P, N, n_words(N), regions, n_regions, swapped);
+  return cuda_fail(cudaGetLastError(), "swap_configs launch");
+}
+
+int launch_swap_values_from_amps(const uint64_t* packed, int64_t P, int N, const uint64_t* regions,
+                                 int n_regions, const float* logabs, const float* sign,
+                                 const float* swapped_logabs, const float* swapped_sign, float* values,
+                                 cudaStream_t s) {
+  if (P == 0 || n_regions == 0) return CGSVMC_OK;
+  swap_values_from_amps_kernel<<<blocks_for(P * n_regions, kThreads), kThreads, 0, s>>>(
+      packed, P, N, n_words(N), regions, n_regions, logabs, sign, swapped_logabs, swapped_sign, values);
+  return cuda_fail(cudaGetLastError(), "swap_values_from_amps launch");
 }
 
 }  // namespace cgsvmc

@@ -3,7 +3,9 @@
 outside the hot path."""
 import collections
 
-from . import distributed, graph_builders
+import torch
+
+from . import distributed, graph_builders, operators
 from .session import Op
 
 EvalOps = collections.namedtuple('EvaluationOps', [
@@ -24,7 +26,8 @@ class MonteCarloOperatorEvaluator(WavefunctionEvaluator):
   def build_eval_ops(self, wavefunction, operator, hparams, shared_resources):
     """evaluation.py:77-110: value = mean of the local values.  An operator
     with a vector local value [B, K] (operators.HeisenbergBonds) gives the
-    float64 numpy vector [K] of the per-column means."""
+    float64 numpy vector [K] of the per-column means; operators.RenyiSwap
+    gives the means over walker pairs [R] (each rank pairs its own shard)."""
     n_sites = hparams.num_sites
     local_batch, walker_id0 = distributed.shard(hparams.batch_size)
     configs = graph_builders.get_configs(shared_resources, local_batch, n_sites,
@@ -34,6 +37,10 @@ class MonteCarloOperatorEvaluator(WavefunctionEvaluator):
 
     def value():
       e = operator.local_value(wavefunction, configs)
+      if isinstance(operator, operators.RenyiSwap):
+        payload = torch.cat([e.double().sum(dim=0), e.new_full((1,), e.shape[0], dtype=torch.float64)])
+        totals = distributed.allreduce_(payload).cpu().numpy()
+        return totals[:-1] / totals[-1]
       if e.dim() == 2:
         totals = distributed.allreduce_(e.double().sum(dim=0))
         return totals.cpu().numpy() / hparams.batch_size

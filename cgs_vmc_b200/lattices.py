@@ -46,6 +46,15 @@ def all_pairs(n_sites):
   return [(i, j) for i in range(n_sites) for j in range(i + 1, n_sites)]
 
 
+def prefix_regions(n_sites):
+  """bool [N // 2, N]: row l - 1 holds sites 0 .. l - 1 (operators.RenyiSwap).
+  On the periodic chain these are the intervals of the S2(l) curve; on the
+  row-major square lattice (s = x * size_y + y) the prefixes of k * size_y
+  sites are cylinders of k rows."""
+  lengths = np.arange(1, n_sites // 2 + 1)
+  return np.arange(n_sites)[None, :] < lengths[:, None]
+
+
 def marshall_signs(n_sites, bonds, j_x, j_z):
   """int8 [N] of +-1: the sublattice signs of the Marshall rotation a
   Hamiltonian was written in.  Bonds with j_x * j_z < 0 are the rotated ones

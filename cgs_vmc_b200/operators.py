@@ -24,7 +24,8 @@ class Operator:
     raise NotImplementedError
 
 
-# values per chunk of walkers in _BondListOperator.bond_values (128 MB of float32)
+# values per chunk of walkers in _BondListOperator.bond_values (128 MB of float32);
+# RenyiSwap keeps its swapped configurations per chunk under the same count
 _BOND_VALUES_CHUNK = 1 << 25
 
 
@@ -158,3 +159,80 @@ class HeisenbergBonds(_BondListOperator):
 
   def apply_in_place(self, wavefunction, inputs, psi=None):
     raise NotImplementedError('HeisenbergBonds has a vector local value only')
+
+
+class RenyiSwap(Operator):
+  """The replica-swap estimator of the second Renyi entropy
+  S2(A) = -log Tr rho_A^2 for every region A of `regions` (bool [R, N]).
+  local_value pairs the walkers (row p with row P + p, P = B // 2; an odd
+  last walker is unused) and returns float32 [P, R]: psi(sigma1')
+  psi(sigma2') / (psi(sigma1) psi(sigma2)) for the pair with its spins in A
+  exchanged, 0 where the replicas hold different numbers of up spins in A
+  (the swapped pair leaves the sampled S^z sector) and exactly 1 where the
+  swap gives back the pair (include/cgsvmc.h, cgsvmc_swap_values).  Its mean
+  is Tr rho_A^2; MonteCarloOperatorEvaluator averages it over pairs."""
+
+  def __init__(self, regions):
+    regions = np.asarray(regions, dtype=bool)
+    if regions.ndim != 2:
+      raise ValueError('regions must be a bool [n_regions, n_sites] array, got shape %s' % (regions.shape,))
+    self.regions = regions
+    self._masks = {}
+
+  def masks(self, device):
+    """int64-viewed uint64 [R, W] site masks on `device` (packed bit convention)."""
+    key = str(device)
+    if key not in self._masks:
+      r, n = self.regions.shape
+      words = np.zeros((r, _native.n_words(n)), dtype=np.uint64)
+      for i in range(n):
+        words[:, i >> 6] |= self.regions[:, i].astype(np.uint64) << np.uint64(i & 63)
+      self._masks[key] = torch.from_numpy(words.view(np.int64)).to(device)
+    return self._masks[key]
+
+  def local_value(self, wavefunction, inputs, psi=None):
+    """float32 [B // 2, R].  A single pure RBM runs the fused kernel; every
+    other wavefunction goes through psi on the swapped pairs.  Pairs are
+    processed in chunks of at most _BOND_VALUES_CHUNK swapped configurations."""
+    from . import graph_builders
+    n = inputs.shape[1]
+    if n != self.regions.shape[1]:
+      raise ValueError('regions have %d sites, the walkers %d' % (self.regions.shape[1], n))
+    packed = graph_builders.as_packed(inputs, n)
+    p = packed.shape[0] // 2
+    masks = self.masks(packed.device)
+    r = masks.shape[0]
+    out = torch.empty(p, r, dtype=torch.float32, device=packed.device)
+    if p == 0 or r == 0:
+      return out
+    fused = None
+    if wavefunction.fast_path:
+      fused = wavefunction.native(n)
+      try:
+        fused.swap_values(packed[:0], masks)       # no pairs: probes for support
+      except NotImplementedError:
+        fused = None
+    else:
+      wavefunction.connect(n)
+    chunk = max(1, _BOND_VALUES_CHUNK // (2 * r))
+    for c0 in range(0, p, chunk):
+      c1 = min(p, c0 + chunk)
+      pc = packed[:2 * p] if c1 - c0 == p else torch.cat([packed[c0:c1], packed[p + c0:p + c1]])
+      oc = out[c0:c1]
+      if fused is not None:
+        fused.swap_values(pc, masks, out=oc)
+        continue
+      logabs, sign = wavefunction.amplitudes(pc)
+      swapped = _native.swap_configs(pc, n, masks)
+      sl, ss = wavefunction.amplitudes(swapped.reshape((c1 - c0) * r * 2, -1))
+      _native.swap_values_from_amps(
+          pc, n, masks, logabs.float().contiguous(), sign.float().contiguous(),
+          sl.float().reshape(c1 - c0, r, 2).contiguous(), ss.float().reshape(c1 - c0, r, 2).contiguous(),
+          out=oc)
+    return out
+
+  def build(self, wavefunction, inputs, psi=None):
+    raise NotImplementedError('RenyiSwap has a per-pair local value only')
+
+  def apply_in_place(self, wavefunction, inputs, psi=None):
+    raise NotImplementedError('RenyiSwap has a per-pair local value only')

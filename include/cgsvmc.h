@@ -247,6 +247,31 @@ int cgsvmc_bond_values(const cgsvmc_ansatz* ansatz, const cgsvmc_ham* ham,
                        const uint64_t* packed, int64_t n_walkers, float* values,
                        void* stream);
 
+/* Replica-swap values of the second Renyi entropy S2(A) = -log Tr rho_A^2.
+ * `packed` holds 2 * n_pairs walkers: pair p is sigma1 = row p and sigma2 =
+ * row n_pairs + p.  `regions` (device, uint64 [n_regions, W]) holds one site
+ * mask per region in the packed bit convention; every mask is ANDed with the
+ * valid-site mask, so bits at or above n_sites are ignored.  With
+ * D = (sigma1 ^ sigma2) & A, the swapped pair is sigma1' = sigma1 ^ D (sigma1
+ * outside A, sigma2 inside) and sigma2' = sigma2 ^ D, and
+ *   values[p, r] = psi(sigma1') psi(sigma2') / (psi(sigma1) psi(sigma2))
+ * (float32 [n_pairs, n_regions], row-major), whose mean over pairs drawn from
+ * |psi|^2 is Tr rho_A^2, with two rules:
+ *   - 0 unless sigma1 and sigma2 hold the same number of up spins in A: the
+ *     sampled state is psi projected on the walkers' S^z sector, whose
+ *     amplitude vanishes on a swapped pair that leaves it;
+ *   - exactly 1.0f when D is empty or holds every site where the replicas
+ *     differ (the swapped pair is the pair itself, possibly exchanged).
+ * A value overflows to +inf where the log ratio exceeds the float32 range;
+ * the estimator is unusable for such a region anyway.  The entropy does not
+ * depend on a Marshall frame (a product of single-site unitaries).
+ * Built for the pure RBM (the shapes of cgsvmc_bond_values); any other ansatz
+ * returns CGSVMC_ERR_UNSUPPORTED, also with n_pairs == 0, so a call without
+ * pairs probes for support.  n_pairs == 0 and n_regions == 0 are no-ops. */
+int cgsvmc_swap_values(const cgsvmc_ansatz* ansatz, const uint64_t* packed,
+                       int64_t n_pairs, const uint64_t* regions,
+                       int32_t n_regions, float* values, void* stream);
+
 /* ---- estimators ------------------------------------------------------- */
 
 /* Replaces the two tf.gradients + accumulators of
@@ -409,6 +434,24 @@ int cgsvmc_bond_values_from_amps(const cgsvmc_ham* ham, const uint64_t* packed,
                                  int64_t n_walkers, const float* logabs,
                                  const float* sign, const float* flipped_logabs,
                                  const float* flipped_sign, float* values,
+                                 void* stream);
+/* The replica swap of cgsvmc_swap_values (same pairs, regions and rules) for
+ * every ansatz.  cgsvmc_swap_configs is its integer half, the counterpart of
+ * cgsvmc_flip_enum: swapped uint64 [n_pairs, n_regions, 2, W] holds sigma1'
+ * then sigma2'.  cgsvmc_swap_values_from_amps takes the amplitudes of the
+ * pairs (logabs, sign float32 [2 n_pairs]) and of the swapped pairs
+ * (swapped_logabs, swapped_sign float32 [n_pairs, n_regions, 2]) and writes
+ *   values[p, r] = sign products * exp(l1' + l2' - l1 - l2)
+ * outside the two rules; sign arrays may be NULL (all +1), so signed outputs
+ * and composites are covered.  Overflows to +inf like cgsvmc_swap_values. */
+int cgsvmc_swap_configs(const uint64_t* packed, int64_t n_pairs, int32_t n_sites,
+                        const uint64_t* regions, int32_t n_regions,
+                        uint64_t* swapped, void* stream);
+int cgsvmc_swap_values_from_amps(const uint64_t* packed, int64_t n_pairs,
+                                 int32_t n_sites, const uint64_t* regions,
+                                 int32_t n_regions, const float* logabs,
+                                 const float* sign, const float* swapped_logabs,
+                                 const float* swapped_sign, float* values,
                                  void* stream);
 
 /* Replaces tf.metrics.mean(local_energy) bookkeeping (training.py:555):

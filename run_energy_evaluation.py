@@ -20,6 +20,9 @@ flags.DEFINE_string('hparams', '', 'Comma-separated name=value overrides.')
 flags.DEFINE_string('correlations_file', '',
                     'Optional .npz for the spin-spin correlations <S_i . S_j> of all site pairs '
                     '(and the structure factor when the lattice geometry is known).')
+flags.DEFINE_string('renyi_file', '',
+                    'Optional .npz for the second Renyi entropy S2 of the prefix regions '
+                    '(sites 0 .. l-1 for l = 1 .. N/2), by the replica-swap estimator.')
 FLAGS = flags.FLAGS
 
 
@@ -58,6 +61,29 @@ def main(argv):
     evaluate_correlations(evaluator, wavefunction, hparams, shared_resources, session, signs,
                           has_bond_file=os.path.exists(os.path.join(FLAGS.checkpoint_dir, 'J.txt')),
                           rank=rank)
+  if FLAGS.renyi_file:
+    evaluate_renyi(evaluator, wavefunction, hparams, shared_resources, session, rank=rank)
+
+
+def evaluate_renyi(evaluator, wavefunction, hparams, shared_resources, session, rank):
+  """S2 = -log Tr rho_A^2 of every prefix region from one more evaluation on
+  the same walkers (replica swap of walker pairs).  The entropy and its error
+  are NaN where the mean swap value is not positive."""
+  regions = lattices.prefix_regions(hparams.num_sites)
+  ops = evaluator.build_eval_ops(wavefunction=wavefunction, operator=operators.RenyiSwap(regions),
+                                 hparams=hparams, shared_resources=shared_resources)
+  samples = np.asarray(evaluator.run_evaluation(ops, session, hparams, epoch_num=0))
+  if rank != 0:
+    return
+  mean = samples.mean(axis=0)
+  stderr = samples.std(axis=0) / np.sqrt(len(samples))
+  positive = mean > 0
+  safe = np.where(positive, mean, 1.0)
+  entropy = np.where(positive, -np.log(safe), np.nan)
+  entropy_stderr = np.where(positive, stderr / safe, np.nan)
+  with open(FLAGS.renyi_file, 'wb') as f:
+    np.savez(f, regions=regions, swap_mean=mean, swap_stderr=stderr, entropy=entropy,
+             entropy_stderr=entropy_stderr)
 
 
 def evaluate_correlations(evaluator, wavefunction, hparams, shared_resources, session, signs, has_bond_file,
